@@ -16,6 +16,9 @@ the other half of the BASELINE metric — is reported in the same line under "b1
     roofline  the acceleration kernel alone against the B200 FP64 peak (20 flop per pair)
     cpu_baseline  the unmodified reference program (oracle/_ref/nbody = samples/nbody.cc) on one host
               core, full b20 run (N=1, rank 0 only)
+
+--dump-outputs DIR writes the state the timed steps left (positions.npy, velocities.npy) so that two builds run
+with the same arguments can be compared output for output: the input system is generated from a fixed seed.
 """
 import argparse
 import importlib
@@ -253,6 +256,21 @@ class ClockSampler:
                 "source": self.source}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_state(np, out_dir, q, v, n):
+    """Planar q[3n] and v[3n] as returned by positions() / velocities(), saved as float64 [3, n] arrays.  Above
+    DUMP_LIMIT_BYTES in all, the same fixed sample of bodies (seed 0, ascending index) is taken from both."""
+    q, v = q.reshape(3, n), v.reshape(3, n)
+    if q.nbytes + v.nbytes > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // (2 * 3 * 8), replace=False))
+        q, v = q[:, keep], v[:, keep]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "positions.npy"), np.ascontiguousarray(q, dtype=np.float64))
+    np.save(os.path.join(out_dir, "velocities.npy"), np.ascontiguousarray(v, dtype=np.float64))
+
+
 def close_states(np, q, v, qo, vo):
     """FAST-math parity bar of SURVEY 8d C5: q within 1e-12*max|v|*dt (or 2 ulp), v within 1e-12 relative.
     Returns (ok, max relative v difference, max absolute q difference)."""
@@ -441,6 +459,10 @@ def run_ours(args):
     dev_ms = max_over_ranks(dev_ms)
     pairs_per_step = n * (n - 1)
     value = pairs_per_step * args.steps / (dev_ms * 1e-3)
+    if args.dump_outputs:
+        q_out, v_out = sh.positions(), sh.velocities()  # every rank: velocities() gathers the shards
+        if rank == 0:
+            dump_state(np, args.dump_outputs, q_out, v_out, n)
 
     # ---- the acceleration kernel alone (roofline) ---------------------------------------------------
     nb.profile_enable(True)
@@ -793,8 +815,15 @@ def main():
                     help="also run the reference's own hw5.cu (rebuilt for sm_100a, needs two visible GPUs) on b1024 as a process")
     ap.add_argument("--cpu-b100-full", action="store_true",
                     help="also time the full b100 run of the unmodified samples/nbody.cc (about 3 minutes of one host core)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of the large workload, write the state they computed to DIR as positions.npy "
+                         "and velocities.npy (float64, planar [3, n]; a fixed sample of bodies above 64 MiB in all)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "large"):
+        ap.error("--dump-outputs applies to the large workload of --impl ours")
     if args.impl == "reference":
         run_reference_arm(args)
     elif args.workload == "ensemble":

@@ -6,6 +6,7 @@ import subprocess
 
 import numpy as np
 import pytest
+from conftest import GOLDEN
 
 
 def test_generator_is_deterministic_and_follows_config_c5(nb):
@@ -43,6 +44,13 @@ def test_nbtool_gen_writes_the_same_file_as_the_library(nb, tmp_path):
     nb.write_input(str(b), nb.generate_system(64, 9, 2))
     assert a.read_bytes() == b.read_bytes()
     assert subprocess.run([nb.NBTOOL_PATH, "frobnicate"], capture_output=True).returncode == 2
+
+
+def test_nbtool_gen_writes_the_stored_vector(nb, tmp_path):
+    """The file the test below feeds to the reference program is pinned byte for byte (generator and writer)."""
+    out = tmp_path / "g.in"
+    subprocess.check_call([nb.NBTOOL_PATH, "gen", "5", "3", str(out), "1"])
+    assert out.read_bytes() == open(os.path.join(GOLDEN, "gen_5_3_1.in"), "rb").read()
 
 
 def test_generated_file_is_a_valid_input_of_the_unmodified_reference(nb, oracle, tmp_path):
