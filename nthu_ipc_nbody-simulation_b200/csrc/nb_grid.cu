@@ -29,7 +29,7 @@
 //     every block publishes step s-1 only after it finished reading step s-2.
 //
 // Warp roles (384 threads = 12 warps: compute warp groups 0-3 and 4-7, helper warp group 8-11; registers are re-allocated
-// between them with setmaxnreg, see NB_GRID_REG_COMPUTE below):
+// between them with setmaxnreg, see REG_COMPUTE below):
 //   * 8 COMPUTE warps = 2 body groups x 4 j-quarters: warp w holds bodies 8c + 4(w>>2) .. +3 in registers and
 //     takes records 128k + 32(w&3) + lane: four i-bodies share every j record read from shared memory
 //     (conflict-free LDS.128 pairs: lanes with bit 2 set read the record's second half first).  A transposing
@@ -44,6 +44,7 @@
 //   * 1 PRODUCER thread: arms the stage's mbarrier with the expected byte count and issues the TMA copies.
 //   * lock-step launches (two systems per launch): 1 INTEGRATOR warp takes the serial tail of a step (sum of the j-parts,
 //     integration, publication) from warp 0, the compute warps only arrive at its barrier and go on to the other system.
+//   * the last warp of the helper warp group is idle.
 //
 // Spins are bounded (clock64) and raise `status`; co-residency comes from the cooperative launch
 // (grid <= SM count, 1 block/SM).
@@ -68,46 +69,31 @@
 #include "nb_internal.h"
 #include "nb_math.cuh"
 
-// Register re-allocation between the warp roles (setmaxnreg, sm_90a+).  With 10 warps two of the four schedulers hold three
-// warps, so no thread can have more than 168 registers, and at 166 ptxas serialises the four pair chains of a record
-// (its own stall counts: 363 cycles per 8 pairs, 416 - 462 in the two-system kernel).  The block is launched with 12 warps
-// instead (the helper warp group 8 - 11: observer, producer, two idle warps), the helpers shrink to NB_GRID_REG_HELPER
-// registers and the eight compute warps grow to NB_GRID_REG_COMPUTE: 320 cycles per 8 pairs, pairs phase 2860 -> 2430 clk
-// (FP64 pipe 76 -> 90 % busy in that phase), b1024 3.38 -> 3.30 us per step, 1-GPU solve 1.23 -> 1.19 s (224 / 56: 3.36 /
-// 1.205, the observer spills; 216 / 72: 3.30 / 1.19; 200 / 104: 3.37 / 1.19).  The pool is what the launch allocated: the
-// increase WAITS until 8 x compute + 4 x helper <= 12 x 168 - a larger request hangs the kernel.  0 = off (10 warps).
-#ifndef NB_GRID_REG_COMPUTE
-#define NB_GRID_REG_COMPUTE 208
-#endif
-#ifndef NB_GRID_REG_HELPER
-#define NB_GRID_REG_HELPER 88
-#endif
-static_assert(NB_GRID_REG_COMPUTE == 0 || (8 * NB_GRID_REG_COMPUTE + 4 * NB_GRID_REG_HELPER <= 12 * 168 && NB_GRID_REG_COMPUTE % 8 == 0 &&
-                                           NB_GRID_REG_HELPER % 8 == 0 && NB_GRID_REG_HELPER >= 24 && NB_GRID_REG_COMPUTE <= 232),
-              "setmaxnreg: the compute warps' increase must fit into what the helper warps release");
-
 namespace nb {
 
 namespace {
 
-constexpr bool REGALLOC = NB_GRID_REG_COMPUTE > 0;
-// With the helper warp group in place (REGALLOC) and several systems in lock step, one of its idle warps is the INTEGRATOR: the
-// compute warps only ARRIVE at the barrier behind their reduction and go on to the next system, the integrator waits there,
-// sums the j-parts, integrates and publishes.  NB_GRID_INTEGRATOR=0 (and always with one system): warp 0 of the compute set.
-#ifndef NB_GRID_INTEGRATOR
-#define NB_GRID_INTEGRATOR 1
-#endif
-#ifndef NB_GRID_UNROLL
-#define NB_GRID_UNROLL 2
-#endif
-constexpr int PAIR_UNROLL = NB_GRID_UNROLL;  // records per trip of the pair loop (4 pairs each)
+// Register re-allocation between the warp roles (setmaxnreg, sm_90a+).  With 10 warps two of the four schedulers hold three
+// warps, so no thread can have more than 168 registers, and at 166 ptxas serialises the four pair chains of a record
+// (its own stall counts: 363 cycles per 8 pairs, 416 - 462 in the two-system kernel).  The block is launched with 12 warps
+// instead (the helper warp group 8 - 11: observer, producer, integrator, idle warp), the helpers shrink to REG_HELPER
+// registers and the eight compute warps grow to REG_COMPUTE: 320 cycles per 8 pairs, pairs phase 2860 -> 2430 clk
+// (FP64 pipe 76 -> 90 % busy in that phase), b1024 3.38 -> 3.30 us per step, 1-GPU solve 1.23 -> 1.19 s (224 / 56: 3.36 /
+// 1.205, the observer spills; 216 / 72: 3.30 / 1.19; 200 / 104: 3.37 / 1.19).  The pool is what the launch allocated: the
+// increase WAITS until 8 x compute + 4 x helper <= 12 x 168 - a larger request hangs the kernel.
+constexpr int REG_COMPUTE = 208, REG_HELPER = 88;
+static_assert(8 * REG_COMPUTE + 4 * REG_HELPER <= 12 * 168 && REG_COMPUTE % 8 == 0 && REG_HELPER % 8 == 0 && REG_HELPER >= 24 &&
+                  REG_COMPUTE <= 232,
+              "setmaxnreg: the compute warps' increase must fit into what the helper warps release");
+
+constexpr int PAIR_UNROLL = 2;   // records per trip of the pair loop (4 pairs each)
 constexpr int GB = 8;            // bodies per block
 constexpr int BPW = 4;           // bodies per compute warp
-constexpr int MAX_NJ = 8;        // compute warps = 2 body groups x NJ j-parts (NJ = 4 or 8); then the observer warp and
-                                 // the producer warp (lane 0 only)
+constexpr int NJ = 4;            // compute warps = 2 body groups x NJ j-parts; then the helper warp group
+constexpr int NTHREADS = 384;    // 8 compute warps + observer, producer (lane 0 only), integrator and idle warp
 constexpr int MAX_T = 2;         // systems per launch (shared memory: 80 B per record each)
 constexpr int MAX_CS = 8;        // largest cluster
-constexpr int RPAD = 32 * MAX_NJ; // shared-memory stages hold a multiple of this many records
+constexpr int RPAD = 256;        // shared-memory stages hold a multiple of this many records (the tail beyond R: zero mass)
 constexpr int FLAG_STOP = 1, FLAG_REDO = 2;
 constexpr long long SPIN_LIMIT = 4000000000LL;  // ~2 s of SM clocks
 constexpr int NPROF = 24;
@@ -167,9 +153,8 @@ __device__ __forceinline__ uint32_t cluster_nctarank() {
     asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
     return r;
 }
-// named barrier of one system's compute warps (id 1 + its warp-set index)
-template <int NTHREADS>
-__device__ __forceinline__ void compute_bar(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "n"(NTHREADS) : "memory"); }
+// named barrier 1: the compute warps
+__device__ __forceinline__ void compute_bar() { asm volatile("bar.sync 1, %0;" ::"n"(32 * 2 * NJ) : "memory"); }
 
 // Record layout: one 32-byte sector {x, y, z, tag}.  The tag is SELF-CHECKING: step in the upper 32 bits, a 32-bit
 // fold of the bit patterns of x, y and z in the lower 32, so a record is accepted only if all four words belong
@@ -216,8 +201,7 @@ struct Shared {
     volatile int abort;
     volatile int delay[MAX_T];      // copy delay after the trigger (clk): a constant, or steered by stale_own (adaptive mode)
     volatile int stale_own[MAX_T];  // this step's validation found stale records in the slice this block's producer copied
-    double iqv[MAX_T][2][32];       // several systems per warp set: position / velocity component of the integrator lanes
-    double part[MAX_T][2][2 * MAX_NJ][3 * BPW];  // per compute warp: sums {ax, ay, az} of its 4 bodies over its j-part ([0] unless SPLIT)
+    double part[MAX_T][2][2 * NJ][3 * BPW];  // per compute warp: sums {ax, ay, az} of its 4 bodies over its j-part
 };
 
 struct ObsState {  // per system, observer warp
@@ -232,16 +216,13 @@ struct ObsState {  // per system, observer warp
 // The validation pass of the compute warps (256 threads, thread tid checks records tid + 256k): every record of the stage
 // must pass the FULL self-check for step `st`.  A record that does not was copied before its publication (stale: the
 // common case, and how the fast blocks wait for the slowest) or is torn: its thread polls that sector in global memory
-// until it passes and patches shared memory.  A function of its own (A/B: -DNB_GRID_VALIDATE_ATTR=__noinline__): the FP64 pair
-// loop's register allocation is sensitive to what is inlined around it (measured on B200, b1024, us per step: validation
-// written inline in the step loop 3.80, this function force-inlined 3.40, out of line 3.49; round 1's tag-only check 3.21).
-#ifndef NB_GRID_VALIDATE_ATTR
-#define NB_GRID_VALIDATE_ATTR __forceinline__
-#endif
-template <int NTHR>
-__device__ NB_GRID_VALIDATE_ATTR bool validate_stage(double* pos, const double* grec, int R, int st, int tid, int hsel, volatile int* abort_flag,
-                                            int* status, unsigned long long* n_stale, int own_lo, int own_hi, volatile int* stale_own) {
+// until it passes and patches shared memory.  A function of its own, force-inlined: the FP64 pair loop's register allocation
+// is sensitive to what is inlined around it (measured on B200, b1024, us per step: validation written inline in the step loop
+// 3.80, this function force-inlined 3.40, out of line 3.49; round 1's tag-only check 3.21).
+__device__ __forceinline__ bool validate_stage(double* pos, const double* grec, int R, int st, int tid, int hsel, volatile int* abort_flag,
+                                               int* status, unsigned long long* n_stale, int own_lo, int own_hi, volatile int* stale_own) {
     bool patched = false;
+    constexpr int NTHR = 32 * 2 * NJ;             // the compute warps
     constexpr int NK = (1024 + NTHR - 1) / NTHR;  // records per thread (n <= 1024)
     double2 va[NK], vb[NK];  // whole records, conflict-free LDS.128 pairs (lanes with bit 2 set read the second half first)
 #pragma unroll
@@ -279,11 +260,9 @@ __device__ NB_GRID_VALIDATE_ATTR bool validate_stage(double* pos, const double* 
 }
 
 // PROFILE: block 0 thread 0 accumulates clock64 per phase (NB_GRID_PROFILE=1)
-// SPLIT (T > 1, NB_GRID_SPLIT=1, off by default: measured slower, see launch_m): every system has its OWN warp set (NJ compute
-// warps that take two j-parts each, an observer warp, a producer thread) and runs at its own pace - two independent "virtual
-// blocks" per SM that share nothing but the FP64 pipe.  Without SPLIT one warp set steps the T systems in turn (lock step).
-template <int MATH, int T, int NJ, bool PROFILE, bool SPLIT>
-__global__ void __launch_bounds__(SPLIT ? 32 * T * (NJ + 2) : (REGALLOC ? 384 : 32 * (2 * NJ + 2)), 1)
+// T systems per launch: one set of compute warps steps them in turn (lock step)
+template <int T, bool PROFILE>
+__global__ void __launch_bounds__(NTHREADS, 1)
 grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ fst, double* __restrict__ gbuf,
                  long long* __restrict__ prof, int* __restrict__ status, int R, int delay_clk, int delay_single, int adapt_up,
                  int adapt_down) {
@@ -292,13 +271,12 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int c = blockIdx.x;
     const int n = descs[0].n;
-    constexpr int PPW = SPLIT ? 2 : 1;  // j-parts per compute warp
-    constexpr int NCW = 2 * NJ / PPW, NSET = SPLIT ? T : 1, W_OBS = NSET * NCW, W_PROD = W_OBS + NSET, RQ = 32 * NJ;
-    constexpr int GT = (REGALLOC && !SPLIT) ? 384 : 32 * (W_PROD + NSET);  // threads of the block (REGALLOC: two idle warps)
-    constexpr int TL = SPLIT ? 1 : T;  // systems per warp set: a role warp handles systems tb .. tb + TL - 1
-    // integrator warp = W_PROD + NSET, for several systems in lock step only: with one system nothing else could use the time, and
-    // the hand-over costs it 130 clk per step (measured: 3.30 -> 3.43 us; two systems: 1-GPU solve 1.18 -> 1.14 s)
-    constexpr bool USE_INT = REGALLOC && !SPLIT && TL > 1 && NB_GRID_INTEGRATOR;
+    constexpr int NCW = 2 * NJ, W_OBS = NCW, W_PROD = W_OBS + 1, W_INT = W_PROD + 1, RQ = 32 * NJ;
+    // With several systems in lock step, warp W_INT is the INTEGRATOR: the compute warps only ARRIVE at the barrier behind their
+    // reduction and go on to the next system, the integrator waits there, sums the j-parts, integrates and publishes (two systems:
+    // 1-GPU solve 1.18 -> 1.14 s).  With one system nothing else could use the time, and the hand-over costs it 130 clk per step
+    // (measured: 3.30 -> 3.43 us), so warp 0 of the compute warps integrates.
+    constexpr bool USE_INT = T > 1;
     constexpr int BAR_INT = 2;  // named barriers BAR_INT + t: the compute warps arrive, the integrator waits (32 * (NCW + 1) threads)
     const int RS = (R + RPAD - 1) / RPAD * RPAD;  // records per stage in shared memory (tail beyond R: zero mass, never copied)
     // per system: pos[2][RS] records {x, y, z, tag} then gm[2][RS]
@@ -340,7 +318,7 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
         double* g0 = s_gm(t, sb & 1);
         double* g1 = s_gm(t, (sb & 1) ^ 1);
         const double f1 = fst[sb + 1];
-        for (int r = tid; r < RS; r += GT) {
+        for (int r = tid; r < RS; r += NTHREADS) {
             double x = 0, y = 0, z = 0, ga = 0, gb = 0;
             if (r < n) {
                 x = d.q[r], y = d.q[r + n], z = d.q[r + 2 * n];
@@ -405,36 +383,34 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
 
     // two branches, each behind its own setmaxnreg (warp-group aligned: warps 0-3 and 4-7 compute, 8-11 help)
     if (warp >= W_OBS) {
-#if NB_GRID_REG_COMPUTE > 0
-    if (!SPLIT) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(NB_GRID_REG_HELPER));
-#endif
-    if (USE_INT && warp == W_PROD + NSET) {
+    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REG_HELPER));
+    if (USE_INT && warp == W_INT) {
         // ------------------------------------------------------------------ INTEGRATOR warp (lane < 24: body 8c + lane/3, component lane%3)
         const int ib = lane / 3, ik = lane - 3 * ib, my_body = c * GB + ib;
         const bool integ = lane < 3 * GB, mine = integ && my_body < n;
-        int istep[TL], ibegin[TL], iend[TL];
-        bool iact[TL];
-        double iq[TL], iv[TL];
+        int istep[T], ibegin[T], iend[T];
+        bool iact[T];
+        double iq[T], iv[T];
         bool any = false;
 #pragma unroll
-        for (int u = 0; u < TL; u++) {
-            const TrajDesc& d = descs[u];
-            istep[u] = ibegin[u] = d.step_begin, iend[u] = d.step_end;
-            iact[u] = !((d.kind >= NB_KIND_Q2) && d.ev->hit_step != -2);
-            iq[u] = mine ? d.q[ik * n + my_body] : 0.0;
-            iv[u] = mine ? d.v[ik * n + my_body] : 0.0;
-            any |= iact[u];
+        for (int t = 0; t < T; t++) {
+            const TrajDesc& d = descs[t];
+            istep[t] = ibegin[t] = d.step_begin, iend[t] = d.step_end;
+            iact[t] = !((d.kind >= NB_KIND_Q2) && d.ev->hit_step != -2);
+            iq[t] = mine ? d.q[ik * n + my_body] : 0.0;
+            iv[t] = mine ? d.v[ik * n + my_body] : 0.0;
+            any |= iact[t];
         }
         bool aborted = false;
         while (any && !aborted) {
 #pragma unroll
-            for (int u = 0; u < TL; u++) {
-                if (!iact[u]) continue;
-                const int t = u, st = istep[u], stage = st & 1;
+            for (int t = 0; t < T; t++) {
+                if (!iact[t]) continue;
+                const int st = istep[t], stage = st & 1;
                 // the observer's verdict on step st, as the compute warps read it: on STOP they do not come to the barrier
-                const int flags = wait_bar(&sh.obs[t][stage], (uint32_t)((st - ibegin[u]) >> 1) & 1u) ? (int)sh.flags[t][stage] : (int)FLAG_STOP;
+                const int flags = wait_bar(&sh.obs[t][stage], (uint32_t)((st - ibegin[t]) >> 1) & 1u) ? (int)sh.flags[t][stage] : (int)FLAG_STOP;
                 if (flags & FLAG_STOP) {
-                    iact[u] = false;
+                    iact[t] = false;
                     continue;
                 }
                 asm volatile("bar.sync %0, %1;" ::"r"(BAR_INT + t), "n"(32 * (NCW + 1)) : "memory");  // the eight warps' sums are in sh.part
@@ -449,56 +425,53 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
                     double a = p[0];
 #pragma unroll
                     for (int j = 1; j < NJ; j++) a += p[j * 3 * BPW];  // fixed order: deterministic
-                    if (my_body < n) kick_drift(a, iv[u], iq[u]);
+                    if (my_body < n) kick_drift(a, iv[t], iq[t]);
                 }
-                const double qy = __shfl_down_sync(0xffffffffu, iq[u], 1);
-                const double qz = __shfl_down_sync(0xffffffffu, iq[u], 2);
-                if (integ && ik == 0) st_sector(g_rec(t, st + 1) + 4 * (size_t)my_body, iq[u], qy, qz, make_tag(st + 1, iq[u], qy, qz));
-                istep[u] = st + 1;
+                const double qy = __shfl_down_sync(0xffffffffu, iq[t], 1);
+                const double qz = __shfl_down_sync(0xffffffffu, iq[t], 2);
+                if (integ && ik == 0) st_sector(g_rec(t, st + 1) + 4 * (size_t)my_body, iq[t], qy, qz, make_tag(st + 1, iq[t], qy, qz));
+                istep[t] = st + 1;
             }
             any = false;
 #pragma unroll
-            for (int u = 0; u < TL; u++) any |= iact[u];
+            for (int t = 0; t < T; t++) any |= iact[t];
         }
         if (mine) {
 #pragma unroll
-            for (int u = 0; u < TL; u++) {
-                descs[u].q[ik * n + my_body] = iq[u];
-                descs[u].v[ik * n + my_body] = iv[u];
+            for (int t = 0; t < T; t++) {
+                descs[t].q[ik * n + my_body] = iq[t];
+                descs[t].v[ik * n + my_body] = iv[t];
             }
         }
-    } else if (warp >= W_PROD + NSET) {
-        // idle warp(s) of the helper warp group (REGALLOC only)
+    } else if (warp >= W_INT) {
+        // idle: the last warp of the helper warp group, and the integrator's with one system
     } else if (warp >= W_PROD) {
         // ------------------------------------------------------------------ PRODUCER thread
-        const int tb = SPLIT ? warp - W_PROD : 0;
         if (lane == 0) {
             const uint32_t CS = cluster_nctarank(), rank = cluster_ctarank();
             const uint32_t slice = (uint32_t)R / CS;  // records per cluster rank (R is a multiple of 8*CS)
             const uint16_t mask = (uint16_t)((1u << CS) - 1u);
-            int pstep[TL];
-            bool pact[TL];
+            int pstep[T];
+            bool pact[T];
             bool any = false;
 #pragma unroll
-            for (int u = 0; u < TL; u++) {
-                const int t = tb + u;
-                pstep[u] = descs[t].step_begin;
-                pact[u] = !sh.stop[t] && descs[t].step_end > descs[t].step_begin;
-                any |= pact[u];
+            for (int t = 0; t < T; t++) {
+                pstep[t] = descs[t].step_begin;
+                pact[t] = !sh.stop[t] && descs[t].step_end > descs[t].step_begin;
+                any |= pact[t];
             }
             while (any && !sh.abort) {
                 any = false;
 #pragma unroll
-                for (int u = 0; u < TL; u++) {
-                    const int t = tb + u;
-                    if (!pact[u]) continue;
-                    const int st = pstep[u] + 1;
+                for (int t = 0; t < T; t++) {
+                    if (!pact[t]) continue;
+                    const int st = pstep[t] + 1;
                     // wait (hardware-suspended on the mbarrier, no issue slots taken from the compute warps) until this
                     // block's sums of step st are complete: it publishes within ~150 clk, and so does everybody
                     bool go = wait_bar(&sh.trig[t][st & 1], (uint32_t)((st - descs[t].step_begin - 1) >> 1) & 1u);
                     if (sh.stop[t]) go = false;
                     if (!go) {
-                        pact[u] = false;
+                        pact[t] = false;
                         continue;
                     }
                     const long long t1 = clock64();
@@ -508,10 +481,10 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
                     // copy reads them.  The blocks keep in step only through the data; whoever copies too early finds stale
                     // tags and polls (validation below), so the delay is a speed knob, not a correctness condition.
                     int dl = adapt_up > 0 ? sh.delay[t] : delay_clk;
-                    if (TL > 1 && adapt_up <= 0) {  // the only system still running in this launch waits for every copy: shortest delay
+                    if (T > 1 && adapt_up <= 0) {  // the only system still running in this launch waits for every copy: shortest delay
                         int n_act = 0;
 #pragma unroll
-                        for (int w = 0; w < TL; w++) n_act += pact[w] ? 1 : 0;
+                        for (int w = 0; w < T; w++) n_act += pact[w] ? 1 : 0;
                         if (n_act == 1) dl = delay_single;
                     }
                     while (clock64() - t1 < dl) {
@@ -522,22 +495,20 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
                         tma_load(dst, src, slice * 32u, bar);
                     else
                         tma_load_multicast(dst, src, slice * 32u, bar, mask);
-                    pstep[u] = st;
-                    if (st >= descs[t].step_end) pact[u] = false;
-                    any |= pact[u];
+                    pstep[t] = st;
+                    if (st >= descs[t].step_end) pact[t] = false;
+                    any |= pact[t];
                 }
             }
         }
     } else {
         // ------------------------------------------------------------------ OBSERVER warp
-        const int tb = SPLIT ? warp - W_OBS : 0;
-        ObsState os[TL];
+        ObsState os[T];
         bool any = false;
 #pragma unroll
-        for (int u = 0; u < TL; u++) {
-            const int t = tb + u;
+        for (int t = 0; t < T; t++) {
             const TrajDesc& d = descs[t];
-            ObsState& s = os[u];
+            ObsState& s = os[t];
             s.n_dev = d.n_dev, s.kind = d.kind, s.DD = d.destroy_device;
             s.Prec = d.planet, s.Arec = d.asteroid;
             s.DDrec = (s.DD >= 0 && s.DD < n) ? s.DD : 0;
@@ -561,9 +532,8 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
         while (any && !sh.abort) {
             any = false;
 #pragma unroll
-            for (int u = 0; u < TL; u++) {
-                const int t = tb + u;
-                ObsState& s = os[u];
+            for (int t = 0; t < T; t++) {
+                ObsState& s = os[t];
                 if (!s.active) continue;
                 const int st = s.step, stage = st & 1;
                 if (st > s.step_begin && !wait_bar(&sh.full[t][stage], (uint32_t)((st - s.step_begin - 1) >> 1) & 1u)) {
@@ -632,9 +602,9 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
         // events (block 0 reports; every block computed the same)
         if (c == 0) {
 #pragma unroll
-            for (int u = 0; u < TL; u++) {
-                const TrajDesc& d = descs[tb + u];
-                ObsState& s = os[u];
+            for (int t = 0; t < T; t++) {
+                const TrajDesc& d = descs[t];
+                ObsState& s = os[t];
 #pragma unroll
                 for (int h = 0; h < 2; h++)
                     if (lane + 32 * h < s.n_dev) d.ev->reach_step[lane + 32 * h] = s.my_reach[h];
@@ -652,24 +622,19 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
         }
     }
     } else {
-#if NB_GRID_REG_COMPUTE > 0
-        if (!SPLIT) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(NB_GRID_REG_COMPUTE));
-#endif
+        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REG_COMPUTE));
         // ------------------------------------------------------------------ COMPUTE warps
-        const int tb = SPLIT ? warp / NCW : 0;          // the warp set's (first) system
-        const int cw = warp - tb * NCW, ctid = tid - tb * 32 * NCW;  // warp / thread index inside the set
-        const int bar_id = 1 + tb;
-        const int bg = cw / (NJ / PPW), part0 = (cw % (NJ / PPW)) * PPW;  // body group, first j-part
+        const int bg = warp / NJ, part0 = warp % NJ;  // body group, j-part
         const int body0 = c * GB + bg * BPW;  // the warp's four bodies (records body0 .. body0+3)
         const int hsel = (lane >> 2) & 1;     // conflict-free LDS.128 pairs: these lanes read the second half first
-        // integrator threads (warp 0 of the set, lane < 24): body 8c + lane/3, component lane%3
+        // integrator threads of one system (warp 0, lane < 24): body 8c + lane/3, component lane%3
         const int ib = lane / 3, ik = lane - 3 * ib;
         const int my_body = c * GB + ib;
-        const bool integ = cw == 0 && lane < 3 * GB;
+        const bool integ = warp == 0 && lane < 3 * GB;
 
-        int cstep[TL], cbegin[TL], cend[TL];
-        bool cact[TL];
-        double iq[TL], iv[TL];
+        int cstep[T], cbegin[T], cend[T];
+        bool cact[T];
+        double iq = 0.0, iv = 0.0;  // one system: position / velocity component of the integrator threads
         long long pacc[6] = {0, 0, 0, 0, 0, 0}, pt = 0;
         unsigned long long n_stale = 0;
         auto tick = [&](int phase) {
@@ -681,15 +646,16 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
         };
         bool any = false;
 #pragma unroll
-        for (int u = 0; u < TL; u++) {
-            const TrajDesc& d = descs[tb + u];
-            cstep[u] = cbegin[u] = d.step_begin, cend[u] = d.step_end;
-            cact[u] = !((d.kind >= NB_KIND_Q2) && d.ev->hit_step != -2);
-            const bool mine = integ && my_body < n;
-            iq[u] = mine ? d.q[ik * n + my_body] : 0.0;
-            iv[u] = mine ? d.v[ik * n + my_body] : 0.0;
-            if (TL > 1 && cw == 0) sh.iqv[tb + u][0][lane] = iq[u], sh.iqv[tb + u][1][lane] = iv[u];
-            any |= cact[u];
+        for (int t = 0; t < T; t++) {
+            const TrajDesc& d = descs[t];
+            cstep[t] = cbegin[t] = d.step_begin, cend[t] = d.step_end;
+            cact[t] = !((d.kind >= NB_KIND_Q2) && d.ev->hit_step != -2);
+            if (!USE_INT) {
+                const bool mine = integ && my_body < n;
+                iq = mine ? d.q[ik * n + my_body] : 0.0;
+                iv = mine ? d.v[ik * n + my_body] : 0.0;
+            }
+            any |= cact[t];
         }
         long long g0 = 0, c0 = 0;
         if (PROFILE) {
@@ -700,14 +666,13 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
 
         while (any && !aborted) {
 #pragma unroll
-            for (int u = 0; u < TL; u++) {
-                const int t = tb + u;
-                if (!cact[u]) continue;  // uniform across the grid
+            for (int t = 0; t < T; t++) {
+                if (!cact[t]) continue;  // uniform across the grid
                 if (PROFILE) pt = clock64();
-                const int st = cstep[u], stage = st & 1;
-                const bool last = st >= cend[u];
+                const int st = cstep[t], stage = st & 1;
+                const bool last = st >= cend[t];
                 // a failed wait has raised sh.abort: the warps still meet at this step's barriers and leave together below
-                if (!last && st > cbegin[u]) wait_bar(&sh.full[t][stage], (uint32_t)((st - cbegin[u] - 1) >> 1) & 1u);
+                if (!last && st > cbegin[t]) wait_bar(&sh.full[t][stage], (uint32_t)((st - cbegin[t] - 1) >> 1) & 1u);
                 tick(0);
                 double* pos = s_pos(t, stage);
                 const double* cg = s_gm(t, stage);
@@ -723,12 +688,12 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
                     const int own_lo = (int)cluster_ctarank() * (R / (int)cluster_nctarank());
                     // (measured worse with two systems in lock step: warps 1-7 validating while warp 0 still integrates and
                     // publishes the other system - 1.31 s against 1.27 s for the b1024 solve on one GPU)
-                    const bool patched = validate_stage<32 * NCW>(pos, grec, R, st, ctid, hsel, &sh.abort, status, &n_stale, own_lo,
-                                                                  own_lo + R / (int)cluster_nctarank(), &sh.stale_own[t]);
+                    const bool patched = validate_stage(pos, grec, R, st, tid, hsel, &sh.abort, status, &n_stale, own_lo,
+                                                        own_lo + R / (int)cluster_nctarank(), &sh.stale_own[t]);
                     // generic-proxy writes to a buffer the async proxy (TMA) overwrites two steps later
                     if (patched) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                    compute_bar<32 * NCW>(bar_id);
-                    if (adapt_up > 0 && ctid == 0) {
+                    compute_bar();
+                    if (adapt_up > 0 && tid == 0) {
                         // closed loop on the copy delay: stale records in the slice this block's producer copied = it copied
                         // too early (raise the delay by adapt_up); a clean step lowers it by adapt_down.  The slowest
                         // block never sees stale records, so ITS delay - the one on the critical path - decays to the floor.
@@ -762,7 +727,7 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
                             const double jx = hsel ? B.x : A.x, jy = hsel ? B.y : A.y, jz = hsel ? A.x : B.x;
                             const double jg = cg[r];
 #pragma unroll
-                            for (int i = 0; i < BPW; i++) pair<MATH>(xi[i], yi[i], zi[i], jx, jy, jz, jg, ax[i], ay[i], az[i]);
+                            for (int i = 0; i < BPW; i++) pair<MATH_FAST>(xi[i], yi[i], zi[i], jx, jy, jz, jg, ax[i], ay[i], az[i]);
                         }
                     }
                 };
@@ -797,76 +762,57 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
                     }
                 };
                 for (int attempt = 0; attempt < 2; attempt++) {
-                    if (PPW == 1) {
-                        pairs_part(part0);
-                        tick(1);
-                    } else {
-                        // a warp of a SPLIT set takes PPW j-parts one after the other, each summed and reduced exactly as a
-                        // warp of the 8-warp set does it: the arithmetic (and so every bit of the state) is the same
-#pragma unroll 1
-                        for (int pp = 0; pp < PPW; pp++) {
-                            pairs_part(part0 + pp);
-                            tick(1);
-                            butterfly_store(part0 + pp);
-                            tick(3);
-                        }
-                    }
+                    pairs_part(part0);
+                    tick(1);
                     // (2) the observer's verdict on the positions of step st
-                    flags = wait_bar(&sh.obs[t][stage], (uint32_t)((st - cbegin[u]) >> 1) & 1u) ? sh.flags[t][stage] : 0;
+                    flags = wait_bar(&sh.obs[t][stage], (uint32_t)((st - cbegin[t]) >> 1) & 1u) ? sh.flags[t][stage] : 0;
                     if (!(flags & FLAG_REDO)) break;  // else: the device was destroyed at this very step, once per trajectory
                 }
                 tick(2);
                 if (flags & FLAG_STOP) {
-                    cact[u] = false;
-                    if (ctid == 0) {  // releases the producer, which waits for the trigger of step st + 1
+                    cact[t] = false;
+                    if (tid == 0) {  // releases the producer, which waits for the trigger of step st + 1
                         sh.stop[t] = 1;
                         __threadfence_block();
                         mbar_arrive(&sh.trig[t][(st + 1) & 1]);
                     }
                     continue;
                 }
-                if (PPW == 1) butterfly_store(part0);
+                butterfly_store(part0);
                 tick(3);
                 if (USE_INT)  // the integrator warp takes it from here
                     asm volatile("bar.arrive %0, %1;" ::"r"(BAR_INT + t), "n"(32 * (NCW + 1)) : "memory");
                 else
-                    compute_bar<32 * NCW>(bar_id);
+                    compute_bar();
                 if (sh.abort) {  // an exchange wait timed out somewhere in this block
                     aborted = true;
                     break;
                 }
                 // (4) warp 0: a = sum of the j-parts; v += a*dt; q += v*dt (nbody.cc:77-88); publish the body as one
                 //     tagged sector {x, y, z, step}, unfenced
-                if (!USE_INT && cw == 0) {
+                if (!USE_INT && warp == 0) {
                     if (lane == 0) mbar_arrive(&sh.trig[t][(st + 1) & 1]);  // producer trigger: everybody publishes within ~150 clk
                     if (integ) {
                         const double* p = &sh.part[t][stage][(ib >> 2) * NJ][3 * (ib & 3) + ik];
                         double a = p[0];
 #pragma unroll
                         for (int j = 1; j < NJ; j++) a += p[j * 3 * BPW];  // fixed order: deterministic
-                        if (TL > 1) {  // state of the other systems stays out of the pair loop's registers
-                            double q_ = sh.iqv[t][0][lane], v_ = sh.iqv[t][1][lane];
-                            if (my_body < n) kick_drift(a, v_, q_);
-                            sh.iqv[t][0][lane] = q_, sh.iqv[t][1][lane] = v_;
-                            iq[0] = q_;
-                        } else if (my_body < n)
-                            kick_drift(a, iv[u], iq[u]);
+                        if (my_body < n) kick_drift(a, iv, iq);
                     }
-                    const double qx = TL > 1 ? iq[0] : iq[u];
-                    const double qy = __shfl_down_sync(0xffffffffu, qx, 1);
-                    const double qz = __shfl_down_sync(0xffffffffu, qx, 2);
-                    if (integ && ik == 0) st_sector(g_rec(t, st + 1) + 4 * (size_t)my_body, qx, qy, qz, make_tag(st + 1, qx, qy, qz));
+                    const double qy = __shfl_down_sync(0xffffffffu, iq, 1);
+                    const double qz = __shfl_down_sync(0xffffffffu, iq, 2);
+                    if (integ && ik == 0) st_sector(g_rec(t, st + 1) + 4 * (size_t)my_body, iq, qy, qz, make_tag(st + 1, iq, qy, qz));
                 }
-                cstep[u] = st + 1;
+                cstep[t] = st + 1;
                 tick(4);
             }
             any = false;
 #pragma unroll
-            for (int u = 0; u < TL; u++) any |= cact[u];
+            for (int t = 0; t < T; t++) any |= cact[t];
         }
-        if (aborted && ctid == 0) {
+        if (aborted && tid == 0) {
 #pragma unroll
-            for (int u = 0; u < TL; u++) sh.stop[tb + u] = 1;
+            for (int t = 0; t < T; t++) sh.stop[t] = 1;
         }
 
         if (PROFILE) {
@@ -879,14 +825,10 @@ grid_traj_kernel(const TrajDesc* __restrict__ descs, const double* __restrict__ 
             }
         }
         if (PROFILE && n_stale) atomicAdd((unsigned long long*)&prof[5], n_stale);
-        // write back
+        // write back (several systems: the integrator warp)
         if (!USE_INT && integ && my_body < n) {
-#pragma unroll
-            for (int u = 0; u < TL; u++) {
-                const TrajDesc& d = descs[tb + u];
-                d.q[ik * n + my_body] = TL > 1 ? sh.iqv[tb + u][0][lane] : iq[u];
-                d.v[ik * n + my_body] = TL > 1 ? sh.iqv[tb + u][1][lane] : iv[u];
-            }
+            descs[0].q[ik * n + my_body] = iq;
+            descs[0].v[ik * n + my_body] = iv;
         }
     }
     if (PROFILE && tid == 0) {  // globaltimer at the end of this block's work: prof[10] = min, prof[11] = max
@@ -923,9 +865,8 @@ WsLayout ws_layout(int n, int T) {
     return w;
 }
 
-template <int MATH, int T, int NJ, bool SPLIT = false>
+template <int T>
 int launch_t(int n, int cs, const TrajDesc* descs, const double* fst, void* ws, cudaStream_t stream) {
-    constexpr int GT = SPLIT ? 32 * T * (NJ + 2) : (REGALLOC ? 384 : 32 * (2 * NJ + 2));
     const int C = padded_blocks(n, cs);
     const size_t smem = smem_for(n, T, cs);
     const WsLayout w = ws_layout(n, MAX_T);  // one layout for every T: the status word has a fixed place
@@ -938,10 +879,9 @@ int launch_t(int n, int cs, const TrajDesc* descs, const double* fst, void* ws, 
     // 1100; on another box 750 gave 3.9 and 900 gave 3.2, so 900 it is); with two systems in lock step the copy of one hides
     // behind the pair loop of the other and a longer delay (fewer stale records, fewer polls) wins (measured: b1024
     // four-trajectory solve on one GPU 2.33 s at 900, 2.00 s at 2600)
-    // SPLIT: every system has its own warp set and timeline, i.e. behaves like a single system
-    static const int delay_clk_env = (T == 1 || SPLIT) ? env_int("NB_GRID_DELAY", 900) : env_int("NB_GRID_DELAY2", 3000);
+    static const int delay_clk_env = T == 1 ? env_int("NB_GRID_DELAY", 900) : env_int("NB_GRID_DELAY2", 3000);
     static const int delay_single_env = env_int("NB_GRID_DELAY", 900);
-    auto kern = profile ? grid_traj_kernel<MATH, T, NJ, true, SPLIT> : grid_traj_kernel<MATH, T, NJ, false, SPLIT>;
+    auto kern = profile ? grid_traj_kernel<T, true> : grid_traj_kernel<T, false>;
     NB_CUDA(cudaMemsetAsync(ws, 0, w.gbuf_bytes, stream));  // tag 0 = no step
     if (profile) NB_CUDA(cudaMemsetAsync(prof, 0, NPROF * sizeof(long long), stream));
 
@@ -956,7 +896,7 @@ int launch_t(int n, int cs, const TrajDesc* descs, const double* fst, void* ws, 
     }
     int R = C * GB, delay_clk = delay_clk_env, delay_single = delay_single_env;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(C), cfg.blockDim = dim3(GT), cfg.dynamicSmemBytes = smem, cfg.stream = stream;
+    cfg.gridDim = dim3(C), cfg.blockDim = dim3(NTHREADS), cfg.dynamicSmemBytes = smem, cfg.stream = stream;
     cudaLaunchAttribute attrs[2];
     attrs[0].id = cudaLaunchAttributeClusterDimension;
     attrs[0].val.clusterDim.x = cs, attrs[0].val.clusterDim.y = 1, attrs[0].val.clusterDim.z = 1;
@@ -1005,12 +945,11 @@ int launch_t(int n, int cs, const TrajDesc* descs, const double* fst, void* ws, 
         return true;
     }();
     (void)adapt_read;
-    // two systems in lock step (T > 1, not SPLIT): the copy of one system hides behind the other's step, so the delay is a
-    // constant in the middle of that window (NB_GRID_DELAY2) - measured on B200, b1024 three-query solve on one GPU: adaptive
-    // (capped at 1600 clk) 1.45 s with 36 000 stale records per step, constant 2600: 1.33 - 1.40 s, 3400: 1.32 s with 170,
-    // 5000: 1.39 s, 7000: 1.78 s; NB_GRID_ADAPT2=1 turns the closed loop on there too
-    static const int adapt2 = env_int("NB_GRID_ADAPT2", 0);
-    const int a_up = (T == 1 || SPLIT || adapt2) ? adapt_up : 0;
+    // two systems in lock step: the copy of one system hides behind the other's step, so the delay is a constant in the
+    // middle of that window (NB_GRID_DELAY2) - measured on B200, b1024 three-query solve on one GPU: adaptive (capped at
+    // 1600 clk) 1.45 s with 36 000 stale records per step, constant 2600: 1.33 - 1.40 s, 3400: 1.32 s with 170, 5000: 1.39 s,
+    // 7000: 1.78 s
+    const int a_up = T == 1 ? adapt_up : 0;
     NB_CUDA(cudaLaunchKernelEx(&cfg, kern, descs, fst, gbuf, prof, status, R, delay_clk, delay_single, a_up, adapt_down));
     count_launch();
     {
@@ -1037,20 +976,6 @@ int launch_t(int n, int cs, const TrajDesc* descs, const double* fst, void* ws, 
     return NB_OK;
 }
 
-template <int MATH>
-int launch_m(int T, int n, int cs, const TrajDesc* descs, const double* fst, void* ws, cudaStream_t stream) {
-    if (T == 1) return launch_t<MATH, 1, 4>(n, cs, descs, fst, ws, stream);
-    // Two systems per launch: one set of 8 compute warps steps both in turn (lock step: the exchange of one system hides
-    // behind the other's step).  NB_GRID_SPLIT=1: each system has its own set of 4 compute warps, observer and producer and
-    // runs at its own pace - same arithmetic, same results; measured SLOWER (b1024 three-query solve on one GPU 1.35 - 1.46 s
-    // against 1.27 s): one compute warp per scheduler keeps the FP64 pipe only 33 % busy (ncu: 49 % of its pair-loop samples
-    // wait on fixed-latency dependencies, 17 % on MUFU.RSQ64H), two warps of the same system 76 %, so two half-speed systems
-    // side by side do not beat two full-speed systems in turn (profiles/r02_grid_exchange.md, section 5).
-    static const int split = env_int("NB_GRID_SPLIT", 0);
-    if (split) return launch_t<MATH, 2, 4, true>(n, cs, descs, fst, ws, stream);
-    return launch_t<MATH, 2, 4>(n, cs, descs, fst, ws, stream);
-}
-
 // cluster size: NB_GRID_CS (1, 2, 4, 8), default 4; every cluster must be co-resident
 int cluster_size_for(int n) {
     static const int want = env_int("NB_GRID_CS", 4);
@@ -1070,7 +995,7 @@ static int group_size(int n, int cs) {
     return T < cap ? T : (cap < 1 ? 1 : cap);
 }
 
-bool grid_traj_supported(int gpu, int n, int n_traj) {
+bool grid_traj_supported(int gpu, int n) {
     static const int enabled = env_int("NB_GRID", 1);
     static const int min_n = env_int("NB_GRID_MIN_N", 128);
     if (!enabled || n < min_n || n > NB_MAX_SMALL_N) return false;
@@ -1103,16 +1028,14 @@ bool grid_traj_supported(int gpu, int n, int n_traj) {
 
 void grid_traj_warm() {
     cudaFuncAttributes fa;
-    (void)cudaFuncGetAttributes(&fa, grid_traj_kernel<MATH_FAST, 1, 4, false, false>);
-    (void)cudaFuncGetAttributes(&fa, grid_traj_kernel<MATH_FAST, 2, 4, false, false>);  // two systems in lock step (default)
+    (void)cudaFuncGetAttributes(&fa, grid_traj_kernel<1, false>);
+    (void)cudaFuncGetAttributes(&fa, grid_traj_kernel<2, false>);  // two systems in lock step
 }
 
 // device address of the status word of a workspace: 0 = ok, 1 = an exchange spin timed out (read after the stream is idle)
 const int* grid_traj_status(const void* ws, int n) { return (const int*)((const char*)ws + ws_layout(n, MAX_T).gbuf_bytes); }
 
-size_t grid_traj_workspace_bytes(int n, int n_traj) {
-    return ws_layout(n, MAX_T).total;
-}
+size_t grid_traj_workspace_bytes(int n) { return ws_layout(n, MAX_T).total; }
 
 int launch_grid_traj(int math, int n, int n_traj, const TrajDesc* descs, const double* fst, int gpu, void* ws,
                      size_t ws_bytes, cudaStream_t stream) {
@@ -1125,9 +1048,13 @@ int launch_grid_traj(int math, int n, int n_traj, const TrajDesc* descs, const d
     for (int cs = cluster_size_for(n);; cs >>= 1) {
         const int G = group_size(n, cs);
         int rc = NB_OK;
-        for (int t0 = 0; t0 < n_traj && rc == NB_OK; t0 += G) {  // groups of up to G trajectories run in lock step
+        // Groups of up to G trajectories: two systems per launch run in lock step, one set of 8 compute warps steps both in
+        // turn (the exchange of one system hides behind the other's step).  A warp set per system, each at its own pace, was
+        // measured slower (b1024 three-query solve on one GPU 1.35 - 1.46 s against 1.27 s): one compute warp per scheduler
+        // keeps the FP64 pipe only 33 % busy, two warps of the same system 76 % (profiles/r02_grid_exchange.md, section 5).
+        for (int t0 = 0; t0 < n_traj && rc == NB_OK; t0 += G) {
             const int T = n_traj - t0 < G ? n_traj - t0 : G;
-            rc = launch_m<MATH_FAST>(T, n, cs, descs + t0, fst, ws, stream);
+            rc = T == 1 ? launch_t<1>(n, cs, descs + t0, fst, ws, stream) : launch_t<2>(n, cs, descs + t0, fst, ws, stream);
             if (rc == NB_ERR_UNSUPPORTED && t0 > 0) return NB_ERR_CUDA;  // cannot happen: the first group decides
         }
         if (rc != NB_ERR_UNSUPPORTED || cs == 1) return rc;

@@ -218,8 +218,8 @@ struct DeviceBatch {
         // the grid kernel's observer warp keeps two devices per lane (NB_MAX_DEVICES = 64); STRICT needs the single block's
         // ascending-j sum
         bool grid = false;
-        if (allow_grid && math == NB_MATH_FAST && max_dev <= 64 && grid_traj_supported(gpu, n, S)) {
-            size_t need = grid_traj_workspace_bytes(n, S);
+        if (allow_grid && math == NB_MATH_FAST && max_dev <= 64 && grid_traj_supported(gpu, n)) {
+            size_t need = grid_traj_workspace_bytes(n);
             if (need > grid_ws_bytes) {
                 if (grid_ws) NB_CUDA(cudaFree(grid_ws));
                 NB_CUDA(cudaMalloc(&grid_ws, need));

@@ -48,9 +48,9 @@ int traj_js_for(int math, int n);
 // nb_grid.cu: one trajectory batch spread over the whole GPU (cooperative persistent kernel)
 int launch_grid_traj(int math, int n, int n_traj, const TrajDesc* descs_dev, const double* fst_dev, int gpu,
                      void* workspace_dev, size_t workspace_bytes, cudaStream_t stream);
-size_t grid_traj_workspace_bytes(int n, int n_traj);
+size_t grid_traj_workspace_bytes(int n);
 const int* grid_traj_status(const void* workspace_dev, int n);  // sticky status word, read it once the stream is idle
-bool grid_traj_supported(int gpu, int n, int n_traj);
+bool grid_traj_supported(int gpu, int n);
 void grid_traj_warm();  // loads the kernels' module on the current device (lazy loading would do it at the first launch)
 
 }  // namespace nb

@@ -35,18 +35,16 @@ def test_only_sm_100a_cubins(sass):
 def test_grid_kernel_instructions(sass):
     _, funcs = sass
     grid = {k: v for k, v in funcs.items() if "grid_traj_kernel" in k}
-    assert len(grid) >= 4
+    assert len(grid) == 4  # one and two systems per launch, each with and without the phase profile
     for name, body in grid.items():
         assert "UBLKCP" in body and "MULTICAST" in body, name      # TMA bulk copy, multicast into the cluster
         assert "ENL2.256" in body, name                             # one 32-byte sector per record access
         assert "UCGABAR" in body, name                              # cluster barrier around the multicast lifetime
         assert "MUFU.RSQ64H" in body and "DFMA" in body, name
-    # one warp set (not SPLIT): registers re-allocated between compute and helper warps
-    lock = [v for k, v in grid.items() if k.endswith("Lb0EEEvPKNS_8TrajDescEPKdPdPxPiiiiii") or "ELb0EEEv" in k]
-    assert lock and all(b.count("USETMAXREG") == 2 for b in lock)
+        assert body.count("USETMAXREG") == 2, name                  # registers re-allocated between compute and helper warps
     # two systems in lock step: the compute warps arrive at the integrator warp's barrier
-    two = [v for k, v in grid.items() if "ILi0ELi2ELi4ELb0ELb0" in k]
-    assert two and "BAR.ARV" in two[0]
+    two = [v for k, v in grid.items() if "grid_traj_kernelILi2E" in k]
+    assert len(two) == 2 and all("BAR.ARV" in b for b in two)
 
 
 def test_no_tensor_core_or_library_kernels(sass):
@@ -75,7 +73,7 @@ def test_grid_pair_loop_schedule_did_not_regress():
     obj = os.path.join(ROOT, "nthu_ipc_nbody-simulation_b200", "_build", "nb_grid.o")
     if not os.path.exists(obj):
         pytest.skip("object file not kept")
-    for inst in ("ILi0ELi1ELi4ELb0ELb0", "ILi0ELi2ELi4ELb0ELb0"):
+    for inst in ("grid_traj_kernelILi1ELb0E", "grid_traj_kernelILi2ELb0E"):
         out = subprocess.check_output([sys.executable, os.path.join(ROOT, "tools", "sass_loop_stalls.py"), obj, inst, "120"]).decode()
         loops = [(int(m.group(1)), int(m.group(2))) for m in re.finditer(r"(\d+) FP64, sum of stall counts (\d+)", out)]
         pair_loops = [s for n, s in loops if n == 128]  # 8 pairs x 16 FP64 instructions per trip
