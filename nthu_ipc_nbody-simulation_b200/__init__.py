@@ -76,21 +76,6 @@ ABI_SYMBOLS = [
     "nb_sym_pairs", "nb_sym_wait_positions", "nb_sym_step", "nb_sym_step_phase", "nb_sym_plan_describe", "nb_sym_rows", "nb_sym_row_size", "nb_sym_row_stride", "nb_device_warm", "nb_hw5_narrow_visible_gpus", "nb_sym_publish_rows", "nb_sym_unpack_rows", "nb_sym_step_host",
 ]
 
-class _Missing:
-    def __call__(self, *a):
-        raise NbodyError(NB_ERR_UNSUPPORTED, "entry point missing in this build of the library")
-
-
-class _Tolerant:
-    def __init__(self, L):
-        object.__setattr__(self, "_L", L)
-
-    def __getattr__(self, name):
-        try:
-            return getattr(self._L, name)
-        except AttributeError:
-            return _Missing()
-
 
 _lib_handle = None
 _dp = C.POINTER(C.c_double)
@@ -107,8 +92,6 @@ def lib():
         raise ImportError("libnbody_b200.so is not built: run `python -c 'import __graft_entry__ as g; g.build()'` "
                           "(or make -C %s/csrc); there is no CPU fallback" % _HERE)
     L = C.CDLL(LIB_PATH)
-    if os.environ.get("NB_LIB_TOLERANT"):  # tools only: A/B runs against an older build that lacks newer entry points
-        L = _Tolerant(L)
     L.nb_version.restype = C.c_char_p
     L.nb_strerror.restype = C.c_char_p
     L.nb_strerror.argtypes = [C.c_int]

@@ -471,8 +471,58 @@ int nb_ensemble_run(int gpu, int math, int kind, int n_systems, int n, double* q
 }
 
 // ---- the step operator -------------------------------------------------------------------------------
-int nb_large_run_steps_host(int gpu, int math, int n, double* q, double* v, const double* m,
-                            const unsigned char* is_device, int step_begin, int step_end);  // nb_large.cu
+// n > NB_MAX_SMALL_N on one GPU, all bodies local, host buffers in and out.  FAST takes the symmetric stepper (nb_sym.cu:
+// every unordered pair once), STRICT the row kernel (nb_large.cu: one j split, the reference's ascending-j sum).  The
+// first failing call's code is returned; everything is freed on every path.
+static int run_steps_large(int gpu, int math, int n, double* q, double* v, const double* m, const unsigned char* is_device,
+                           int step_begin, int step_end) {
+    NB_CUDA(cudaSetDevice(gpu));
+    const bool sym = math == NB_MATH_FAST;
+    nb_sym* h = nullptr;
+    int rc = sym ? nb_sym_create(n, 1, 0, &h) : NB_OK;
+    if (rc) return rc;
+    cudaStream_t st = nullptr;
+    double *dq = nullptr, *dv = nullptr, *dm = nullptr, *pos[2] = {nullptr, nullptr};
+    unsigned char* ddev = nullptr;
+    void* work = nullptr;  // the symmetric stepper's PJ buffer, or the row kernel's j-split scratch
+    auto chk = [&](cudaError_t e, const char* what) {
+        if (e != cudaSuccess && rc == NB_OK) rc = nb::cuda_fail(e, what, __FILE__, __LINE__);
+    };
+    chk(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking), "cudaStreamCreate");
+    chk(cudaMalloc(&dq, 3 * (size_t)n * sizeof(double)), "cudaMalloc q");
+    chk(cudaMalloc(&dv, 3 * (size_t)n * sizeof(double)), "cudaMalloc v");
+    chk(cudaMalloc(&dm, (size_t)n * sizeof(double)), "cudaMalloc m");
+    chk(cudaMalloc(&ddev, (size_t)n), "cudaMalloc is_device");
+    chk(cudaMalloc(&pos[0], 4 * (size_t)n * sizeof(double)), "cudaMalloc pos4");
+    chk(cudaMalloc(&pos[1], 4 * (size_t)n * sizeof(double)), "cudaMalloc pos4");
+    const size_t work_bytes = (size_t)(sym ? nb_sym_pj_bytes(h) : nb_large_scratch_bytes(n, n));
+    chk(cudaMalloc(&work, work_bytes), sym ? "cudaMalloc PJ" : "cudaMalloc scratch");
+    if (rc == NB_OK && sym) chk(cudaMemsetAsync(work, 0, work_bytes, st), "memset PJ");
+    if (rc == NB_OK) {
+        chk(cudaMemcpyAsync(dq, q, 3 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D q");
+        chk(cudaMemcpyAsync(dv, v, 3 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D v");
+        chk(cudaMemcpyAsync(dm, m, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D m");
+        chk(cudaMemcpyAsync(ddev, is_device, (size_t)n, cudaMemcpyHostToDevice, st), "H2D is_device");
+    }
+    if (rc == NB_OK) rc = nb_large_pack(math, n, dq, dm, ddev, step_begin + 1, pos[0], st);
+    int cur = 0;
+    for (int step = step_begin + 1; step <= step_end && rc == NB_OK; step++) {
+        double *next = pos[cur ^ 1], *pj = (double*)work;
+        rc = sym ? nb_sym_step(h, step, pos[cur], &next, &pj, nullptr, nullptr, dv, dm, ddev, st)
+                 : nb_large_step(math, step, n, 0, n, pos[cur], next, dv, dm, ddev, work, st);
+        cur ^= 1;
+    }
+    if (rc == NB_OK) rc = nb_large_unpack(n, pos[cur], dq, st);
+    if (rc == NB_OK) {
+        chk(cudaMemcpyAsync(q, dq, 3 * (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H q");
+        chk(cudaMemcpyAsync(v, dv, 3 * (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H v");
+        chk(cudaStreamSynchronize(st), "sync");
+    }
+    cudaFree(dq), cudaFree(dv), cudaFree(dm), cudaFree(ddev), cudaFree(pos[0]), cudaFree(pos[1]), cudaFree(work);
+    if (st) cudaStreamDestroy(st);
+    if (h) nb_sym_destroy(h);
+    return rc;
+}
 
 int nb_run_steps(int gpu, int math, int n, double* q, double* v, const double* m, const unsigned char* is_device,
                  int step_begin, int step_end) {
@@ -480,7 +530,7 @@ int nb_run_steps(int gpu, int math, int n, double* q, double* v, const double* m
     if (math != NB_MATH_FAST && math != NB_MATH_STRICT) return NB_ERR_ARG;
     int rc = nb::check_gpu(gpu);
     if (rc) return rc;
-    if (n > NB_MAX_SMALL_N) return nb_large_run_steps_host(gpu, math, n, q, v, m, is_device, step_begin, step_end);
+    if (n > NB_MAX_SMALL_N) return run_steps_large(gpu, math, n, q, v, m, is_device, step_begin, step_end);
     DeviceBatch b;
     rc = b.init(gpu, 1, n, math);
     if (!rc) rc = b.set_system(0, q, v, m, is_device, 0, 0, NB_KIND_PLAIN, -1, step_begin);

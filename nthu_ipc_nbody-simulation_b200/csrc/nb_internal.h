@@ -33,6 +33,9 @@ void count_launch(int n = 1);
 // nb_profile_enable / nb_profile_read (nb_large.cu): event pairs around the acceleration kernel, calling thread only
 bool profile_on();
 void profile_push(cudaEvent_t e0, cudaEvent_t e1);
+// nb_large.cu: stream-ordered wait until counters[0 .. count) all reach target; a wait that times out writes code to *status
+int launch_counter_wait(const unsigned long long* counters, int count, unsigned long long target, int* status, int code,
+                        cudaStream_t stream);
 
 // per-GPU |sin(step*dt/6000)| table (host glibc sin: nbody.cc:14-16 with t = step*dt, nbody.cc:63),
 // entries 0..len-1, built lazily and grown on demand.  Returns a device pointer valid for the

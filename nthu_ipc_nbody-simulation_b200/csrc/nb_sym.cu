@@ -17,19 +17,15 @@
 //     split in half for even P), local work first, so that the peers' positions arrive behind it.
 #include <algorithm>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <mutex>
 #include <vector>
 
+#include "nb_async.cuh"
 #include "nb_internal.h"
 #include "nb_math.cuh"
 #include "nb_sym.cuh"
-
-#ifndef NB_SYM_UNROLL
-#define NB_SYM_UNROLL 2
-#endif
 
 namespace nb {
 namespace sym {
@@ -92,8 +88,6 @@ void spans_of_rank(int n, int world, int p, int sb, std::vector<std::vector<Span
 // i-bodies per lane for this shard size: fewest register slots x relative cost of the loop (measured, n = 65536: 2.93 ms
 // with 6 per lane, 3.00 ms with 8)
 int choose_ipl(int n, int world) {
-    static const int forced = getenv("NB_SYM_I") ? atoi(getenv("NB_SYM_I")) : 0;
-    if (forced == IPL_A || forced == IPL_B) return forced;
     if (n < 1 || world < 1 || n % world) return IPL_A;
     const int S = n / world;
     const double ca = (double)rows_of(S, sb_of(IPL_A)) * sb_of(IPL_A) * 1.0, cb = (double)rows_of(S, sb_of(IPL_B)) * sb_of(IPL_B) * 1.025;
@@ -249,47 +243,12 @@ int build_plan(int n, int world, int rank, int blocks, int ipl, Plan& P) {
 namespace {
 
 constexpr int NT = 32 * WARPS;  // threads per block
-constexpr int ROT_UNROLL = NB_SYM_UNROLL;
+constexpr int ROT_UNROLL = 2;  // unrolled 1 / 4: 2.99 / 2.95 ms per step against 2.93 (profiles/r02_sym_accel.md)
 constexpr int TILE_BYTES = TJ * 32;
 constexpr int STG_DOUBLES = WARPS * 3 * TJ;  // one staging buffer
 constexpr size_t SMEM_BYTES = (size_t)STAGES * TILE_BYTES + 2 * (size_t)STG_DOUBLES * sizeof(double);
 // counter block of a rank (unsigned long long): [kind: 0 = pos4 rows arrived, 1 = partial accelerations arrived][parity][source rank]
 constexpr int CTR_WORDS = 2 * 2 * MAX_PEERS;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_1d(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     smem_u32(dst_smem)),
-                 "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ unsigned long long ld_acquire_sys(const unsigned long long* p) {
-    unsigned long long v;
-    asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void red_release_sys(unsigned long long* p) {
-    asm volatile("red.release.sys.global.add.u64 [%0], %1;" ::"l"(p), "l"(1ULL) : "memory");
-}
 
 struct Peers {
     double* pj[MAX_PEERS];                    // PJ of every rank: [rows_global][3][shard]
@@ -356,14 +315,7 @@ __global__ void __launch_bounds__(NT, MIN_BLOCKS) sym_accel_kernel(AccelArgs A, 
         const int src = segs[p_si].src_rank;
         if (A.pos_target && !(seen >> src & 1u)) {
             // rows of another rank: valid once every block of its integrate kernel has stored them here and released
-            const unsigned long long* ctr = peers.counters[peers.my_rank] + (0 * 2 + A.parity_read) * MAX_PEERS + src;
-            const long long t0 = clock64();
-            while (ld_acquire_sys(ctr) < A.pos_target) {
-                if (clock64() - t0 > 20000000000LL) {  // ~10 s: a lost peer must not hang the GPU
-                    *A.status = 1;
-                    break;
-                }
-            }
+            wait_counter(peers.counters[peers.my_rank] + (0 * 2 + A.parity_read) * MAX_PEERS + src, A.pos_target, A.status, 1);
             asm volatile("fence.proxy.async;" ::: "memory");  // the TMA (async proxy) reads what was just acquired
             seen |= 1u << src;
         }
@@ -500,16 +452,8 @@ constexpr int IB = 32, IP = 8;
 __global__ void __launch_bounds__(IB * IP) sym_integrate_kernel(IntegrateArgs A, Peers peers) {
     __shared__ double part[IP][3][IB];
     if (A.acc_target) {
-        if (threadIdx.x < peers.world) {
-            const unsigned long long* ctr = peers.counters[peers.my_rank] + (1 * 2 + A.parity) * MAX_PEERS + threadIdx.x;
-            const long long t0 = clock64();
-            while (ld_acquire_sys(ctr) < A.acc_target) {
-                if (clock64() - t0 > 20000000000LL) {
-                    *A.status = 2;
-                    break;
-                }
-            }
-        }
+        if (threadIdx.x < peers.world)
+            wait_counter(peers.counters[peers.my_rank] + (1 * 2 + A.parity) * MAX_PEERS + threadIdx.x, A.acc_target, A.status, 2);
         __syncthreads();
     }
     const int bx = threadIdx.x % IB, pt = threadIdx.x / IB;
@@ -588,17 +532,6 @@ __global__ void sym_unpack_rows_kernel(const double4* __restrict__ pos4, int sha
     q_own[il] = p.x, q_own[il + shard] = p.y, q_own[il + 2 * shard] = p.z;
 }
 
-// stream-ordered wait until every rank's rows of the last step have arrived (before the host reads the buffer)
-__global__ void sym_wait_kernel(const unsigned long long* counters, unsigned long long target, int* status) {
-    const long long t0 = clock64();
-    while (ld_acquire_sys(counters + threadIdx.x) < target) {
-        if (clock64() - t0 > 20000000000LL) {
-            *status = 3;
-            break;
-        }
-    }
-}
-
 }  // namespace
 }  // namespace sym
 }  // namespace nb
@@ -638,8 +571,6 @@ static int sym_default_blocks(int* out) {
             set_error_detail("symmetric kernel does not fit on this GPU");
             return NB_ERR_UNSUPPORTED;
         }
-        const char* e = getenv("NB_SYM_BLOCKS_PER_SM");
-        if (e && atoi(e) >= 1 && atoi(e) < per_sm) per_sm = atoi(e);
         it = cache.emplace(dev, sms * per_sm).first;
     }
     *out = it->second;
@@ -752,13 +683,10 @@ long long nb_sym_pairs(const nb_sym* h, long long* sym_pairs, long long* oneside
 int nb_sym_wait_positions(nb_sym* h, const unsigned long long* my_counters, int* status_dev, void* stream) {
     if (!h || !my_counters || !status_dev) return NB_ERR_ARG;
     if (h->plan.world == 1 || h->last_step < 0) return NB_OK;
+    // in stream order, until every rank's rows of the last step have arrived (before the host reads the buffer)
     const int par = h->last_step & 1;
-    sym_wait_kernel<<<1, h->plan.world, 0, (cudaStream_t)stream>>>(my_counters + (0 * 2 + par) * MAX_PEERS,
-                                                                  (unsigned long long)h->integrate_blocks * h->pos_pubs[par],
-                                                                  status_dev);
-    count_launch();
-    NB_CUDA(cudaGetLastError());
-    return NB_OK;
+    return launch_counter_wait(my_counters + (0 * 2 + par) * MAX_PEERS, h->plan.world,
+                               (unsigned long long)h->integrate_blocks * h->pos_pubs[par], status_dev, 3, (cudaStream_t)stream);
 }
 
 int nb_sym_step_phase(nb_sym* h, int step, int phases, const double* pos4_cur, double* const* peer_pos4_next,
@@ -894,53 +822,6 @@ int nb_sym_step(nb_sym* h, int step, const double* pos4_cur, double* const* peer
                 const unsigned char* is_device_dev, void* stream) {
     return nb_sym_step_phase(h, step, 3, pos4_cur, peer_pos4_next, peer_pj, peer_counters, status_dev, vel_dev, m0_dev,
                              is_device_dev, stream);
-}
-
-// host-buffer convenience used by nb_run_steps for n > NB_MAX_SMALL_N, FAST math (single GPU, all bodies local)
-int nb_sym_run_steps_host(int gpu, int n, double* q, double* v, const double* m, const unsigned char* is_device,
-                          int step_begin, int step_end) {
-    NB_CUDA(cudaSetDevice(gpu));
-    nb_sym* h = nullptr;
-    int rc = nb_sym_create(n, 1, 0, &h);
-    if (rc) return rc;
-    cudaStream_t st = nullptr;
-    double *dq = nullptr, *dv = nullptr, *dm = nullptr, *pos[2] = {nullptr, nullptr}, *pj = nullptr;
-    unsigned char* ddev = nullptr;
-    auto chk = [&](cudaError_t e, const char* what) {
-        if (e != cudaSuccess && rc == NB_OK) rc = cuda_fail(e, what, __FILE__, __LINE__);
-    };
-    chk(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking), "cudaStreamCreate");
-    chk(cudaMalloc(&dq, 3 * (size_t)n * sizeof(double)), "cudaMalloc q");
-    chk(cudaMalloc(&dv, 3 * (size_t)n * sizeof(double)), "cudaMalloc v");
-    chk(cudaMalloc(&dm, (size_t)n * sizeof(double)), "cudaMalloc m");
-    chk(cudaMalloc(&ddev, (size_t)n), "cudaMalloc is_device");
-    chk(cudaMalloc(&pos[0], 4 * (size_t)n * sizeof(double)), "cudaMalloc pos4");
-    chk(cudaMalloc(&pos[1], 4 * (size_t)n * sizeof(double)), "cudaMalloc pos4");
-    chk(cudaMalloc(&pj, (size_t)nb_sym_pj_bytes(h)), "cudaMalloc PJ");
-    if (rc == NB_OK) chk(cudaMemsetAsync(pj, 0, (size_t)nb_sym_pj_bytes(h), st), "memset PJ");
-    if (rc == NB_OK) {
-        chk(cudaMemcpyAsync(dq, q, 3 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D q");
-        chk(cudaMemcpyAsync(dv, v, 3 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D v");
-        chk(cudaMemcpyAsync(dm, m, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D m");
-        chk(cudaMemcpyAsync(ddev, is_device, (size_t)n, cudaMemcpyHostToDevice, st), "H2D is_device");
-    }
-    if (rc == NB_OK) rc = nb_large_pack(NB_MATH_FAST, n, dq, dm, ddev, step_begin + 1, pos[0], st);
-    int cur = 0;
-    for (int step = step_begin + 1; step <= step_end && rc == NB_OK; step++) {
-        double* next = pos[cur ^ 1];
-        rc = nb_sym_step(h, step, pos[cur], &next, &pj, nullptr, nullptr, dv, dm, ddev, st);
-        cur ^= 1;
-    }
-    if (rc == NB_OK) rc = nb_large_unpack(n, pos[cur], dq, st);
-    if (rc == NB_OK) {
-        chk(cudaMemcpyAsync(q, dq, 3 * (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H q");
-        chk(cudaMemcpyAsync(v, dv, 3 * (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H v");
-        chk(cudaStreamSynchronize(st), "sync");
-    }
-    cudaFree(dq), cudaFree(dv), cudaFree(dm), cudaFree(ddev), cudaFree(pos[0]), cudaFree(pos[1]), cudaFree(pj);
-    if (st) cudaStreamDestroy(st);
-    nb_sym_destroy(h);
-    return rc;
 }
 
 }  // extern "C"

@@ -7,28 +7,19 @@
 namespace nb {
 namespace sym {
 
-// tuning knobs (A/B builds: -DNB_SYM_I=.. -DNB_SYM_WARPS=.. -DNB_SYM_MIN_BLOCKS=.. -DNB_SYM_TJ=..).  Measured on B200 at
-// n = 65536 (profiles/r02_sym_variants.md): 6 i-bodies per lane, 8 warps, ONE block per SM (254 registers: the six pair
-// chains of a rotation interleave instruction by instruction) 2.93 ms/step; 4 per lane at 128 registers, 16 warps/SM
-// (chains serialised by the register budget, 8-cycle dependent stalls) 3.28 ms; 12 warps x 168 registers 3.12 ms.
-#ifndef NB_SYM_WARPS
-#define NB_SYM_WARPS 8
-#endif
-#ifndef NB_SYM_MIN_BLOCKS
-#define NB_SYM_MIN_BLOCKS 1
-#endif
-#ifndef NB_SYM_TJ
-#define NB_SYM_TJ 128
-#endif
-constexpr int WARPS = NB_SYM_WARPS;      // warps per block
-constexpr int MIN_BLOCKS = NB_SYM_MIN_BLOCKS;  // resident blocks per SM the register budget is set for
+// Measured on B200 at n = 65536 (profiles/r02_sym_accel.md, variants): 6 i-bodies per lane, 8 warps, ONE block per SM (254
+// registers: the six pair chains of a rotation interleave instruction by instruction) 2.93 ms/step; 4 per lane at 128
+// registers, 16 warps/SM (chains serialised by the register budget, 8-cycle dependent stalls) 3.28 ms; 12 warps x 168
+// registers 3.12 ms.
+constexpr int WARPS = 8;       // warps per block
+constexpr int MIN_BLOCKS = 1;  // resident blocks per SM the register budget is set for
 // i-bodies per lane: two instantiations of the kernel.  6 (rows of up to 1536 bodies) is the faster loop; 8 (2048) wastes no
 // register slots when the shard is a power of two (8192 bodies per rank at 8 ranks = 4 rows of 2048, against 6 rows of
-// 1366 in 1536 slots).  choose_ipl() takes the one with the smaller slots x cost product; NB_SYM_I overrides.
+// 1366 in 1536 slots).  choose_ipl() takes the one with the smaller slots x cost product.
 constexpr int IPL_A = 6, IPL_B = 8;
 constexpr int sb_of(int ipl) { return WARPS * 32 * ipl; }  // bodies per row (superblock) = i-bodies per block
 constexpr int MAX_SB = sb_of(IPL_B);
-constexpr int TJ = NB_SYM_TJ;            // j bodies per shared-memory tile
+constexpr int TJ = 128;                  // j bodies per shared-memory tile (64 / 256: 3.01 / 2.96 ms per step against 2.93)
 constexpr int STAGES = 3;                // TMA ring depth
 constexpr int SUB = 32;                  // scheduling granularity along j (one warp rotation group)
 constexpr int MAX_PEERS = 16;

@@ -13,7 +13,6 @@
 // Shared memory: xy[2][n] (double2) and zg[2][n] (double2 {z, G*m_eff}), double-buffered by step
 // parity so that a step needs two block barriers:
 //     [device G*m_eff(step) -> zg[cur]]  B  [forces from buf cur; owner integrates -> buf cur^1]  B  [observers]
-#include <cstdlib>
 
 #include "nb_internal.h"
 #include "nb_math.cuh"
@@ -446,9 +445,9 @@ int launch_traj_batch(int math, int n, int n_traj, const TrajDesc* descs, const 
     if (n < 1 || n > NB_MAX_SMALL_N || n_traj < 1) return NB_ERR_ARG;
     if (math == NB_MATH_STRICT) return launch<MATH_STRICT, 1>(n, n_traj, descs, fst, stream);
     if (math != NB_MATH_FAST) return NB_ERR_ARG;
-    // 896 < n <= 1024 (the 1024-body ensemble): the symmetric kernel; NB_TRAJ_SYM=0 keeps the one-sided one
-    static const bool use_sym = !(getenv("NB_TRAJ_SYM") && atoi(getenv("NB_TRAJ_SYM")) == 0);
-    if (use_sym && n > 1024 - TS_G && n <= 1024) return launch_sym(n_traj, descs, fst, stream);
+    // 896 < n <= 1024 (the 1024-body ensemble): the symmetric kernel (DESIGN 4.2: 115 us per step against the one-sided
+    // kernel's 157 us)
+    if (n > 1024 - TS_G && n <= 1024) return launch_sym(n_traj, descs, fst, stream);
     switch (traj_js_for(math, n)) {
         case 1: return launch<MATH_FAST, 1>(n, n_traj, descs, fst, stream);
         case 2: return launch<MATH_FAST, 2>(n, n_traj, descs, fst, stream);

@@ -52,7 +52,7 @@ def test_no_tensor_core_or_library_kernels(sass):
     one of this repository's."""
     out, funcs = sass
     assert not re.search(r"\b(HMMA|IMMA|DMMA|UTCHMMA|UTCQMMA|UTMALDG)\b", out)
-    own = ("traj_kernel", "traj_sym_kernel", "grid_traj_kernel", "large_", "sym_", "dfma_")
+    own = ("traj_kernel", "traj_sym_kernel", "grid_traj_kernel", "large_", "sym_", "counter_wait_kernel", "dfma_")
     assert all(any(o in name for o in own) for name in funcs), [n for n in funcs if not any(o in n for o in own)]
 
 
@@ -63,6 +63,15 @@ def test_symmetric_kernels_use_tma_and_no_atomics_on_the_accumulation(sass):
             assert "UBLKCP" in body and "SHFL.IDX" in body, name
             assert "ATOM" not in body.replace("ATOMS.CAST", ""), name   # partial rows + fixed-order sums, never atomics
             assert len(re.findall(r"\bDFMA\b", body)) >= 400, name
+
+
+def test_large_n_kernels_are_built_in_the_kept_variants_only(sass):
+    """The row kernel exists once per math mode (FAST, STRICT; 4 i-bodies per thread is a constant), the symmetric kernel
+    once per row width (6 and 8 i-bodies per lane, chosen by shard size).  No other variant is built."""
+    _, funcs = sass
+    targs = lambda kernel: sorted(re.search(kernel + r"I(\w+?)EEv", k).group(1) for k in funcs if kernel in k)
+    assert targs("large_accel_kernel") == ["Li0E", "Li1E"], targs("large_accel_kernel")  # <MATH_FAST>, <MATH_STRICT>
+    assert targs("sym_accel_kernel") == ["Li6E", "Li8E"], targs("sym_accel_kernel")
 
 
 def test_grid_pair_loop_schedule_did_not_regress():
