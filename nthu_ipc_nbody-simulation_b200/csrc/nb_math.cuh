@@ -93,6 +93,27 @@ __device__ __forceinline__ void pair_accum_fast(double c, double dx, double dy, 
     az = fma(c, dz, az);
 }
 
+// FAST, one UNORDERED pair: s = |d|^-3 as in pair<> (rsqrt seed + cubic correction), both accelerations (nb_sym.cu,
+// traj_sym_kernel)
+__device__ __forceinline__ void pair_sym(double xi, double yi, double zi, double gmi, double xj, double yj, double zj,
+                                         double gmj, double& aix, double& aiy, double& aiz, double& ajx, double& ajy,
+                                         double& ajz) {
+    const double dx = xj - xi, dy = yj - yi, dz = zj - zi;
+    const double r2 = fma(dx, dx, fma(dy, dy, fma(dz, dz, EPS2)));
+    const double y0 = rsqrt_seed(r2);
+    const double y2 = y0 * y0;
+    const double e = fma(-r2, y2, 1.0);
+    const double p = fma(e, fma(e, 1.875, 1.5), 1.0);
+    const double s = y0 * (y2 * p);
+    const double ci = gmj * s, cj = gmi * s;
+    aix = fma(ci, dx, aix);
+    aiy = fma(ci, dy, aiy);
+    aiz = fma(ci, dz, aiz);
+    ajx = fma(-cj, dx, ajx);
+    ajy = fma(-cj, dy, ajy);
+    ajz = fma(-cj, dz, ajz);
+}
+
 // v += a*dt; q += v*dt (nbody.cc:77-88, hw5.cu:235-236).  O(n) per step, so both math modes keep
 // the reference's four separate roundings (no FMA): the state update is then exactly run_step's.
 __device__ __forceinline__ void kick_drift(double a, double& v, double& q) {

@@ -269,26 +269,6 @@ struct AccelArgs {
     int* status;
 };
 
-// one unordered pair: s = |d|^-3 (rsqrt seed + cubic correction, nb_math.cuh), both accelerations
-__device__ __forceinline__ void pair_sym(double xi, double yi, double zi, double gmi, double xj, double yj, double zj,
-                                         double gmj, double& aix, double& aiy, double& aiz, double& ajx, double& ajy,
-                                         double& ajz) {
-    const double dx = xj - xi, dy = yj - yi, dz = zj - zi;
-    const double r2 = fma(dx, dx, fma(dy, dy, fma(dz, dz, EPS2)));
-    const double y0 = rsqrt_seed(r2);
-    const double y2 = y0 * y0;
-    const double e = fma(-r2, y2, 1.0);
-    const double p = fma(e, fma(e, 1.875, 1.5), 1.0);
-    const double s = y0 * (y2 * p);
-    const double ci = gmj * s, cj = gmi * s;
-    aix = fma(ci, dx, aix);
-    aiy = fma(ci, dy, aiy);
-    aiz = fma(ci, dz, aiz);
-    ajx = fma(-cj, dx, ajx);
-    ajy = fma(-cj, dy, ajy);
-    ajz = fma(-cj, dz, ajz);
-}
-
 __device__ __forceinline__ double rot(double v, int src) { return __shfl_sync(0xffffffffu, v, src); }
 
 template <int I_PER_LANE>
