@@ -98,6 +98,78 @@ static int check_gpu(int gpu) {
     return NB_OK;
 }
 
+// Busy-wait for the stream (or for event e) instead of a blocking synchronize: the blocking wait costs tens of milliseconds
+// of wake-up latency now and then (measured on the B200 boxes), and the chain plan of nb_solve waits every few thousand
+// steps.  (round 2: spin for the first 200 us only, then poll every 20 us - a launch lasts milliseconds to seconds, and a
+// host core at 100 % for all of it bought nothing)
+static int spin_wait(cudaStream_t stream, cudaEvent_t e = nullptr) {
+    const auto w0 = std::chrono::steady_clock::now();
+    for (;;) {
+        cudaError_t qe = e ? cudaEventQuery(e) : cudaStreamQuery(stream);
+        if (qe == cudaSuccess) return NB_OK;
+        if (qe != cudaErrorNotReady) return cuda_fail(qe, e ? "cudaEventQuery" : "cudaStreamQuery", __FILE__, __LINE__);
+        if (std::chrono::steady_clock::now() - w0 > std::chrono::microseconds(200))
+            std::this_thread::sleep_for(std::chrono::microseconds(20));
+    }
+}
+
+// ---- the large-N steppers, one system at a time ----------------------------------------------------------
+// n > NB_MAX_SMALL_N on one GPU, all bodies local.  FAST takes the symmetric stepper (nb_sym.cu: every unordered pair once),
+// STRICT the row kernel (nb_large.cu: one j split, the reference's ascending-j sum).  The stepper owns the two pos4 buffers
+// [n][4], and the symmetric stepper's handle and PJ buffer or the row kernel's j-split scratch; the caller's q stays
+// planar [3][n] and its v is stepped in place.  Used by nb_run_steps and by the query path (DeviceBatch::run).
+struct LargeStepper {
+    int n = 0, math = 0, cur = 0;  // pos[cur] holds the current step
+    nb_sym* h = nullptr;
+    double* pos[2] = {nullptr, nullptr};
+    void* work = nullptr;
+
+    // on the current device; the PJ zero-fill is enqueued on st
+    int init(int n_, int math_, cudaStream_t st) {
+        n = n_, math = math_;
+        if (math == NB_MATH_FAST) {
+            const int rc = nb_sym_create(n, 1, 0, &h);
+            if (rc) return rc;
+        }
+        NB_CUDA(cudaMalloc(&pos[0], 4 * (size_t)n * sizeof(double)));
+        NB_CUDA(cudaMalloc(&pos[1], 4 * (size_t)n * sizeof(double)));
+        const size_t bytes = (size_t)(h ? nb_sym_pj_bytes(h) : nb_large_scratch_bytes(n, n));
+        NB_CUDA(cudaMalloc(&work, bytes));
+        if (h) NB_CUDA(cudaMemsetAsync(work, 0, bytes, st));  // PJ rows nobody writes are summed as zeros
+        return NB_OK;
+    }
+    // planar positions of step step_next - 1 with the masses of step_next: the next step() is step_next, any step
+    int pack(const double* q, const double* m, const unsigned char* is_device, int step_next, cudaStream_t st) {
+        cur = 0;
+        if (h) {
+            const int rc = sym_restart(h);
+            if (rc) return rc;
+        }
+        return nb_large_pack(math, n, q, m, is_device, step_next, pos[0], st);
+    }
+    int step(int s, double* v, const double* m, const unsigned char* is_device, cudaStream_t st) {
+        double *next = pos[cur ^ 1], *pj = (double*)work;
+        const int rc = h ? nb_sym_step(h, s, pos[cur], &next, &pj, nullptr, nullptr, v, m, is_device, st)
+                         : nb_large_step(math, s, n, 0, n, pos[cur], next, v, m, is_device, work, st);
+        if (!rc) cur ^= 1;
+        return rc;
+    }
+    int unpack(double* q, cudaStream_t st) { return nb_large_unpack(n, pos[cur], q, st); }
+    void release() {
+        cudaFree(pos[0]), cudaFree(pos[1]), cudaFree(work);
+        if (h) nb_sym_destroy(h);
+        *this = LargeStepper{};
+    }
+};
+
+// Steps per chunk of the query path on the large-N steppers: the host reads the events between chunks.  A step costs
+// about n^2 (2.95 ms at 65 536 bodies on the B200), so 2^33 / n^2 steps, at least 4 (~12 ms at 65 536 bodies) and at most
+// 512 (below ~4 096 bodies a step is bound by launch latency).
+static int large_chunk(int n) {
+    const long long c = (1LL << 33) / ((long long)n * n);
+    return (int)std::min(512LL, std::max(4LL, c));
+}
+
 // ---- a batch of same-n systems resident on one GPU ---------------------------------------------------
 struct DeviceBatch {
     int gpu = -1, S = 0, n = 0, math = 0;
@@ -117,6 +189,11 @@ struct DeviceBatch {
     std::vector<int> cur_step;
     double gpu_seconds = 0.0;
     long long pairs = 0;
+    // n > NB_MAX_SMALL_N: the steppers, shared by the systems (they are stepped in turn), and the events of the system being
+    // stepped after each of the last two chunks (pinned staging, see run_large)
+    LargeStepper large;
+    nb_events* pin_chunk = nullptr;
+    cudaEvent_t chunk_done[2] = {nullptr, nullptr};
 
     int init(int gpu_, int S_, int n_, int math_) {
         gpu = gpu_, S = S_, n = n_, math = math_;
@@ -136,6 +213,13 @@ struct DeviceBatch {
         h_descs.assign(S, TrajDesc{});
         h_ev.assign(S, nb_events{});
         cur_step.assign(S, 0);
+        if (n > NB_MAX_SMALL_N) {
+            const int rc = large.init(n, math, stream);
+            if (rc) return rc;
+            NB_CUDA(cudaHostAlloc(&pin_chunk, 2 * sizeof(nb_events), cudaHostAllocDefault));
+            NB_CUDA(cudaEventCreateWithFlags(&chunk_done[0], cudaEventDisableTiming));
+            NB_CUDA(cudaEventCreateWithFlags(&chunk_done[1], cudaEventDisableTiming));
+        }
         return NB_OK;
     }
     void release() {
@@ -150,6 +234,11 @@ struct DeviceBatch {
         if (pin_ev) cudaFreeHost(pin_ev);
         if (pin_status) cudaFreeHost(pin_status);
         pin_ev = nullptr, pin_status = nullptr;
+        large.release();
+        if (pin_chunk) cudaFreeHost(pin_chunk);
+        pin_chunk = nullptr;
+        for (cudaEvent_t& e : chunk_done)
+            if (e) cudaEventDestroy(e), e = nullptr;
         if (e0) cudaEventDestroy(e0);
         if (e1) cudaEventDestroy(e1);
         if (stream) cudaStreamDestroy(stream);
@@ -218,7 +307,9 @@ struct DeviceBatch {
         // the grid kernel's observer warp keeps two devices per lane (NB_MAX_DEVICES = 64); STRICT needs the single block's
         // ascending-j sum
         bool grid = false;
-        if (allow_grid && math == NB_MATH_FAST && max_dev <= 64 && grid_traj_supported(gpu, n)) {
+        if (n > NB_MAX_SMALL_N) {
+            rc = run_large();
+        } else if (allow_grid && math == NB_MATH_FAST && max_dev <= 64 && grid_traj_supported(gpu, n)) {
             size_t need = grid_traj_workspace_bytes(n);
             if (need > grid_ws_bytes) {
                 if (grid_ws) NB_CUDA(cudaFree(grid_ws));
@@ -249,18 +340,8 @@ struct DeviceBatch {
         *pin_status = 0;
         pin_status[1] = 0;
         if (grid) NB_CUDA(cudaMemcpyAsync(pin_status, grid_traj_status(grid_ws, n), 2 * sizeof(int), cudaMemcpyDeviceToHost, stream));
-        // Busy-wait instead of cudaStreamSynchronize: the blocking wait costs tens of milliseconds of wake-up latency now
-        // and then (measured on the B200 boxes), and the chain plan of nb_solve comes through here every few thousand steps.
-        // (round 2: spin for the first 200 us only, then poll every 20 us - a launch lasts milliseconds to seconds, and
-        // a host core at 100 % for all of it bought nothing)
-        const auto w0 = std::chrono::steady_clock::now();
-        for (;;) {
-            cudaError_t qe = cudaStreamQuery(stream);
-            if (qe == cudaSuccess) break;
-            if (qe != cudaErrorNotReady) return cuda_fail(qe, "cudaStreamQuery", __FILE__, __LINE__);
-            if (std::chrono::steady_clock::now() - w0 > std::chrono::microseconds(200))
-                std::this_thread::sleep_for(std::chrono::microseconds(20));
-        }
+        rc = spin_wait(stream);
+        if (rc) return rc;
         memcpy(h_ev.data(), pin_ev, S * sizeof(nb_events));
         if (pin_status[1] != 0) g_torn_records += pin_status[1];  // records that failed the full self-check and were fetched again
         if (*pin_status != 0) {
@@ -274,6 +355,39 @@ struct DeviceBatch {
             long long steps = h_ev[s].steps_done - cur_step[s];
             if (steps > 0) pairs += steps * (long long)n * (n - 1);
             cur_step[s] = h_ev[s].steps_done;
+        }
+        return NB_OK;
+    }
+    static bool stopped(const nb_events& e, int kind) { return kind >= NB_KIND_Q2 && e.hit_step != -2; }
+    // n > NB_MAX_SMALL_N: the systems one after another on the large-N steppers, each step followed by the one-warp observer
+    // (large_observe_kernel), step_begin observed first unless it already was.  Steps go out in chunks of large_chunk(n):
+    // while chunk c + 1 runs, the host reads the events after chunk c and enqueues nothing more once the stop event has
+    // fired.  The q, v left in a stopped slot are therefore up to two chunks past the stop, while cur_step (= steps_done) is
+    // the stop step: get_state would not return the state at cur_step there.  Nothing reads it - solve_chain reloads such
+    // a slot, and later runs skip a stopped system - so it is not rewound.
+    int run_large() {
+        const int chunk = large_chunk(n);
+        for (int s = 0; s < S; s++) {
+            const TrajDesc& d = h_descs[s];
+            if (stopped(h_ev[s], d.kind) || h_ev[s].steps_done >= d.step_end) continue;
+            int rc = large.pack(d.q, d.m, d.is_device, d.step_begin + 1, stream);
+            if (!rc) rc = launch_large_observe(d, large.pos[large.cur], d.step_begin, stream);
+            for (int st = d.step_begin, c = 0; !rc && st < d.step_end; c++) {
+                const int end = std::min(st + chunk, d.step_end);
+                while (!rc && st < end) {
+                    rc = large.step(++st, d.v, d.m, d.is_device, stream);
+                    if (!rc) rc = launch_large_observe(d, large.pos[large.cur], st, stream);
+                }
+                if (rc || st >= d.step_end) break;
+                NB_CUDA(cudaMemcpyAsync(pin_chunk + (c & 1), d.ev, sizeof(nb_events), cudaMemcpyDeviceToHost, stream));
+                NB_CUDA(cudaEventRecord(chunk_done[c & 1], stream));
+                if (c > 0) {  // chunk c is queued: read the events after chunk c - 1
+                    rc = spin_wait(stream, chunk_done[(c - 1) & 1]);
+                    if (!rc && stopped(pin_chunk[(c - 1) & 1], d.kind)) break;
+                }
+            }
+            if (!rc) rc = large.unpack(d.q, stream);
+            if (rc) return rc;
         }
         return NB_OK;
     }
@@ -471,20 +585,16 @@ int nb_ensemble_run(int gpu, int math, int kind, int n_systems, int n, double* q
 }
 
 // ---- the step operator -------------------------------------------------------------------------------
-// n > NB_MAX_SMALL_N on one GPU, all bodies local, host buffers in and out.  FAST takes the symmetric stepper (nb_sym.cu:
-// every unordered pair once), STRICT the row kernel (nb_large.cu: one j split, the reference's ascending-j sum).  The
-// first failing call's code is returned; everything is freed on every path.
+// n > NB_MAX_SMALL_N on one GPU (LargeStepper), host buffers in and out.  The first failing call's code is returned;
+// everything is freed on every path.
 static int run_steps_large(int gpu, int math, int n, double* q, double* v, const double* m, const unsigned char* is_device,
                            int step_begin, int step_end) {
     NB_CUDA(cudaSetDevice(gpu));
-    const bool sym = math == NB_MATH_FAST;
-    nb_sym* h = nullptr;
-    int rc = sym ? nb_sym_create(n, 1, 0, &h) : NB_OK;
-    if (rc) return rc;
+    int rc = NB_OK;
     cudaStream_t st = nullptr;
-    double *dq = nullptr, *dv = nullptr, *dm = nullptr, *pos[2] = {nullptr, nullptr};
+    double *dq = nullptr, *dv = nullptr, *dm = nullptr;
     unsigned char* ddev = nullptr;
-    void* work = nullptr;  // the symmetric stepper's PJ buffer, or the row kernel's j-split scratch
+    nb::LargeStepper ls;
     auto chk = [&](cudaError_t e, const char* what) {
         if (e != cudaSuccess && rc == NB_OK) rc = nb::cuda_fail(e, what, __FILE__, __LINE__);
     };
@@ -493,34 +603,24 @@ static int run_steps_large(int gpu, int math, int n, double* q, double* v, const
     chk(cudaMalloc(&dv, 3 * (size_t)n * sizeof(double)), "cudaMalloc v");
     chk(cudaMalloc(&dm, (size_t)n * sizeof(double)), "cudaMalloc m");
     chk(cudaMalloc(&ddev, (size_t)n), "cudaMalloc is_device");
-    chk(cudaMalloc(&pos[0], 4 * (size_t)n * sizeof(double)), "cudaMalloc pos4");
-    chk(cudaMalloc(&pos[1], 4 * (size_t)n * sizeof(double)), "cudaMalloc pos4");
-    const size_t work_bytes = (size_t)(sym ? nb_sym_pj_bytes(h) : nb_large_scratch_bytes(n, n));
-    chk(cudaMalloc(&work, work_bytes), sym ? "cudaMalloc PJ" : "cudaMalloc scratch");
-    if (rc == NB_OK && sym) chk(cudaMemsetAsync(work, 0, work_bytes, st), "memset PJ");
+    if (rc == NB_OK) rc = ls.init(n, math, st);
     if (rc == NB_OK) {
         chk(cudaMemcpyAsync(dq, q, 3 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D q");
         chk(cudaMemcpyAsync(dv, v, 3 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D v");
         chk(cudaMemcpyAsync(dm, m, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D m");
         chk(cudaMemcpyAsync(ddev, is_device, (size_t)n, cudaMemcpyHostToDevice, st), "H2D is_device");
     }
-    if (rc == NB_OK) rc = nb_large_pack(math, n, dq, dm, ddev, step_begin + 1, pos[0], st);
-    int cur = 0;
-    for (int step = step_begin + 1; step <= step_end && rc == NB_OK; step++) {
-        double *next = pos[cur ^ 1], *pj = (double*)work;
-        rc = sym ? nb_sym_step(h, step, pos[cur], &next, &pj, nullptr, nullptr, dv, dm, ddev, st)
-                 : nb_large_step(math, step, n, 0, n, pos[cur], next, dv, dm, ddev, work, st);
-        cur ^= 1;
-    }
-    if (rc == NB_OK) rc = nb_large_unpack(n, pos[cur], dq, st);
+    if (rc == NB_OK) rc = ls.pack(dq, dm, ddev, step_begin + 1, st);
+    for (int step = step_begin + 1; step <= step_end && rc == NB_OK; step++) rc = ls.step(step, dv, dm, ddev, st);
+    if (rc == NB_OK) rc = ls.unpack(dq, st);
     if (rc == NB_OK) {
         chk(cudaMemcpyAsync(q, dq, 3 * (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H q");
         chk(cudaMemcpyAsync(v, dv, 3 * (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H v");
         chk(cudaStreamSynchronize(st), "sync");
     }
-    cudaFree(dq), cudaFree(dv), cudaFree(dm), cudaFree(ddev), cudaFree(pos[0]), cudaFree(pos[1]), cudaFree(work);
+    cudaFree(dq), cudaFree(dv), cudaFree(dm), cudaFree(ddev);
+    ls.release();
     if (st) cudaStreamDestroy(st);
-    if (h) nb_sym_destroy(h);
     return rc;
 }
 
@@ -567,7 +667,6 @@ static bool solve_chain_plan(int n_parts, int n_traj, int math_flags) {
 
 static int solve_jobs(const nb_system* sys, std::vector<int>& devs) {
     if (!sys || !sys->q || !sys->v || !sys->m || !sys->is_device || sys->n < 1) return NB_ERR_ARG;
-    if (sys->n > NB_MAX_SMALL_N) return NB_ERR_UNSUPPORTED;
     if (sys->planet < 0 || sys->planet >= sys->n || sys->asteroid < 0 || sys->asteroid >= sys->n) return NB_ERR_ARG;
     devs.clear();
     for (int i = 0; i < sys->n; i++)

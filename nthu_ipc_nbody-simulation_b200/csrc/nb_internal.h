@@ -36,6 +36,10 @@ void profile_push(cudaEvent_t e0, cudaEvent_t e1);
 // nb_large.cu: stream-ordered wait until counters[0 .. count) all reach target; a wait that times out writes code to *status
 int launch_counter_wait(const unsigned long long* counters, int count, unsigned long long target, int* status, int code,
                         cudaStream_t stream);
+// nb_large.cu: the observers of step `step` of trajectory d on the pos4 records [n][4] the step's integrate kernel wrote
+int launch_large_observe(const TrajDesc& d, double* pos4_dev, int step, cudaStream_t stream);
+// nb_sym.cu: forget the steps of a one-rank handle, so that its next step may be any step (positions repacked by the caller)
+int sym_restart(nb_sym* h);
 
 // per-GPU |sin(step*dt/6000)| table (host glibc sin: nbody.cc:14-16 with t = step*dt, nbody.cc:63),
 // entries 0..len-1, built lazily and grown on demand.  Returns a device pointer valid for the

@@ -22,6 +22,7 @@
 #include "nb_async.cuh"
 #include "nb_internal.h"
 #include "nb_math.cuh"
+#include "nb_observe.cuh"
 
 namespace nb {
 namespace {
@@ -203,6 +204,41 @@ __global__ void large_unpack_kernel(int n, const double4* __restrict__ pos4, dou
     q[i] = p.x, q[i + n] = p.y, q[i + 2 * n] = p.z;
 }
 
+// The observers of step st of one trajectory on the large-N steppers: one warp, launched after the step's integrate kernel,
+// reads the records {x, y, z, G*m_eff(st+1)} it wrote.  Lane l looks after devices l and l + 32 (NB_MAX_DEVICES = 64), as
+// the grid kernel's observer warp does.  A stopped trajectory (Q2/Q3 hit) or an already observed step is left as it is,
+// so steps enqueued past the stop change no event.  The Q3 destroy at st zeroes the device's base mass (Observed::store)
+// and the mass of the record just read: the forces of step st+1 are the first without it (hw5.cu:299-307).
+__global__ void __launch_bounds__(32) large_observe_kernel(const TrajDesc d, double4* __restrict__ pos4, int st) {
+    const int lane = threadIdx.x;
+    Observed ob;
+    ob.load(d.ev);
+    const bool stopped = (d.kind >= NB_KIND_Q2) && ob.hit_step != -2;
+    if (stopped || d.ev->steps_done >= st) return;
+    int my_dev[2], my_reach[2];
+#pragma unroll
+    for (int h = 0; h < 2; h++) {
+        const int k = lane + 32 * h;
+        my_dev[h] = k < d.n_dev ? d.dev_index[k] : -1;
+        my_reach[h] = k < d.n_dev ? d.ev->reach_step[k] : -2;
+    }
+    const int DD = d.destroy_device;
+    const bool armed = q3_armed(d.kind, DD, d.n, d.m);
+    const int seen = observe_step<2>(ob, st, d.kind, d.planet, d.asteroid, armed, armed ? DD : 0, my_dev, my_reach,
+                                     [&](int r, double& x, double& y, double& z) {
+                                         const double4 p = pos4[r];
+                                         x = p.x, y = p.y, z = p.z;
+                                     });
+    __syncwarp();  // every lane has read the events before lane 0 rewrites them
+#pragma unroll
+    for (int h = 0; h < 2; h++)
+        if (lane + 32 * h < d.n_dev) d.ev->reach_step[lane + 32 * h] = my_reach[h];
+    if (lane == 0) {
+        ob.store(d, st);
+        if (seen == OBS_DESTROYED) pos4[DD].w = 0.0;
+    }
+}
+
 // optional per-thread profiling of the acceleration kernel (nb_profile_enable / nb_profile_read)
 struct Prof {
     bool on = false;
@@ -229,6 +265,13 @@ void profile_push(cudaEvent_t e0, cudaEvent_t e1) { g_prof.evs.emplace_back(e0, 
 int launch_counter_wait(const unsigned long long* counters, int count, unsigned long long target, int* status, int code,
                         cudaStream_t stream) {
     counter_wait_kernel<<<1, count, 0, stream>>>(counters, target, status, code);
+    count_launch();
+    NB_CUDA(cudaGetLastError());
+    return NB_OK;
+}
+
+int launch_large_observe(const TrajDesc& d, double* pos4_dev, int step, cudaStream_t stream) {
+    large_observe_kernel<<<1, 32, 0, stream>>>(d, (double4*)pos4_dev, step);
     count_launch();
     NB_CUDA(cudaGetLastError());
     return NB_OK;

@@ -531,6 +531,16 @@ struct nb_sym {
     int first_step = -1, last_step = -1, accel_step = -1;
 };
 
+// One rank has no arrival counters: the step bookkeeping only enforces consecutive steps, and a restart may forget it.
+// With world > 1 the counters of every rank count the steps, so there is no restart.
+int nb::sym_restart(nb_sym* h) {
+    if (!h || h->plan.world != 1) return NB_ERR_ARG;
+    h->steps_done[0] = h->steps_done[1] = 0;
+    h->pos_pubs[0] = h->pos_pubs[1] = 0;
+    h->first_step = h->last_step = h->accel_step = -1;
+    return NB_OK;
+}
+
 static int sym_default_blocks(int* out) {
     static std::mutex mu;
     static std::map<int, int> cache;
