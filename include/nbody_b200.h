@@ -130,6 +130,35 @@ int nb_traj_fork(nb_traj* t, int kind, int destroy_device, nb_traj** out);
 int nb_traj_fork_on(nb_traj* t, int gpu, int kind, int destroy_device, nb_traj** out);
 int nb_traj_destroy(nb_traj* t);
 
+/* ---- diagnostics -----------------------------------------------------------------------------
+ * For a state (q, v) at step k, let m_i be the effective mass at t = k*dt: the base mass, with the device rule
+ * m0 + 0.5*m0*|sin(k*dt/6000)| (nbody.cc:14-16, 63) applied to gravity devices, |sin| from the same host glibc
+ * expression as the library's |sin| table.  Any k >= 0 is allowed, not only table entries.
+ *   mass                = sum m_i
+ *   kinetic             = 1/2 sum m_i |v_i|^2
+ *   potential           = -sum_{i<j} G m_i m_j / sqrt(|q_i - q_j|^2 + eps^2): the potential whose gradient is the
+ *                         softened force of nbody.cc:65-72; self pairs are excluded, as the reference skips j == i
+ *   momentum[3]         = sum m_i v_i
+ *   angular_momentum[3] = sum m_i q_i x v_i, about the origin
+ * Under the semi-implicit Euler step of nbody.cc:77-88 with pairwise central forces and constant gravitating masses
+ * (device-free systems, every Q1 trajectory) momentum and angular momentum are conserved exactly in exact arithmetic;
+ * the drift of kinetic + potential is the usual quality measure of a run.
+ * One evaluation (no math argument): r^-1 by the rsqrt seed and a second-order correction, sums in a fixed order with
+ * no atomics, so the result is bit-identical from call to call and independent of the other systems of a batch.  Each
+ * quantity is within a few hundred u = 2^-53 of sum |terms| (DESIGN.md 4.6 states the bound). */
+typedef struct nb_diag {
+    int step, n;
+    double mass, kinetic, potential;
+    double momentum[3], angular_momentum[3];
+} nb_diag;
+/* host arrays, system-major as nb_ensemble_run: q[s][3n], v[s][3n], m[s][n], is_device[s][n]; any n >= 1; out[n_systems].
+ * gpu_seconds (may be NULL) = device time of the diagnostic kernels (CUDA events). */
+int nb_diagnostics(int gpu, int n_systems, int n, const double* q, const double* v, const double* m,
+                   const unsigned char* is_device, int step, nb_diag* out, double* gpu_seconds);
+/* the handle's device-resident state at its current step, with the masses the trajectory now sees
+   (Q1: devices massless; Q3: the destroyed device zeroed); q, v never go to the host */
+int nb_traj_diagnostics(nb_traj* t, nb_diag* out);
+
 /* ---- ensembles ------------------------------------------------------------------------------
  * n_systems independent systems of the same n in one launch, one thread block per system
  * (north-star (c): batches of synthetic systems).  Arrays are system-major: q[s][3*n] ...

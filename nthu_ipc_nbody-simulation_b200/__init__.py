@@ -64,6 +64,19 @@ class NbAnswer(C.Structure):
                 ("n_trajectories", C.c_int), ("n_gpus_used", C.c_int)]
 
 
+class NbDiag(C.Structure):
+    _fields_ = [("step", C.c_int), ("n", C.c_int), ("mass", C.c_double), ("kinetic", C.c_double),
+                ("potential", C.c_double), ("momentum", C.c_double * 3), ("angular_momentum", C.c_double * 3)]
+
+    def as_dict(self):
+        return dict(step=self.step, n=self.n, mass=self.mass, kinetic=self.kinetic, potential=self.potential,
+                    energy=self.kinetic + self.potential, momentum=list(self.momentum),
+                    angular_momentum=list(self.angular_momentum))
+
+
+DIAG_TILE = 256  # tile edge of the diagnostics' pair kernel (nb_internal.h DIAG_T)
+
+
 # every symbol include/nbody_b200.h declares (tests/test_abi.py checks the two lists agree)
 ABI_SYMBOLS = [
     "nb_version", "nb_strerror", "nb_last_error_detail", "nb_device_count", "nb_kernel_launches", "nb_grid_torn_records",
@@ -74,6 +87,7 @@ ABI_SYMBOLS = [
     "nb_dev_alloc", "nb_dev_free", "nb_dev_copy", "nb_ipc_export", "nb_ipc_open", "nb_ipc_close", "nb_fp64_peak", "nb_fp64_peak_variant",
     "nb_sym_create", "nb_sym_destroy", "nb_sym_pj_bytes", "nb_sym_counter_bytes", "nb_sym_blocks", "nb_sym_remote_partial_bytes",
     "nb_sym_pairs", "nb_sym_wait_positions", "nb_sym_step", "nb_sym_step_phase", "nb_sym_plan_describe", "nb_sym_rows", "nb_sym_row_size", "nb_sym_row_stride", "nb_device_warm", "nb_hw5_narrow_visible_gpus", "nb_sym_publish_rows", "nb_sym_unpack_rows", "nb_sym_step_host",
+    "nb_diagnostics", "nb_traj_diagnostics",
 ]
 
 
@@ -162,6 +176,8 @@ def lib():
                                        C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     L.nb_sym_rows.argtypes = [C.c_int, C.c_int]
     L.nb_sym_row_stride.argtypes = [C.c_int, C.c_int]
+    L.nb_diagnostics.argtypes = [C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, _up, C.c_int, C.POINTER(NbDiag), _dp]
+    L.nb_traj_diagnostics.argtypes = [C.c_void_p, C.POINTER(NbDiag)]
     L.nb_fp64_peak.argtypes = [C.c_int, _dp, _dp]
     L.nb_fp64_peak_variant.argtypes = [C.c_int, C.c_int, _dp]
     _lib_handle = L
@@ -298,6 +314,13 @@ class Trajectory:
         _check(lib().nb_traj_state(self._h, _d(q), _d(v), _d(m), C.byref(step)))
         return q, v, m, step.value
 
+    def diagnostics(self):
+        """Mass, energies, momentum and angular momentum of the device-resident state at the current step, with the masses
+        the trajectory now sees (Q1: devices massless; Q3: the destroyed device zeroed).  Returns a dict (NbDiag.as_dict)."""
+        d = NbDiag()
+        _check(lib().nb_traj_diagnostics(self._h, C.byref(d)))
+        return d.as_dict()
+
     def fork(self, kind, destroy_device=-1, gpu=None):
         h = C.c_void_p()
         if gpu is None:
@@ -318,6 +341,28 @@ class Trajectory:
             self.close()
         except Exception:
             pass
+
+
+def diagnostics(q, v, m, is_device, step=0, gpu=0, return_seconds=False):
+    """Mass, kinetic and potential energy, momentum and angular momentum of planar states at `step` (effective device
+    masses of that step; include/nbody_b200.h states the definitions).  q, v: [3n] or [S, 3n]; m, is_device: [n] or
+    [S, n].  Returns a dict for one system, a list of dicts for [S, 3n]; with return_seconds also the device time."""
+    q = np.ascontiguousarray(q, dtype=np.float64)
+    one = q.ndim == 1
+    q = q.reshape(1, -1) if one else q
+    S, n3 = q.shape
+    n = n3 // 3
+    if n3 != 3 * n or n < 1:
+        raise ValueError("q must be [3n] or [S, 3n] with n >= 1")
+    v = np.ascontiguousarray(v, dtype=np.float64).reshape(S, 3 * n)
+    m = np.ascontiguousarray(m, dtype=np.float64).reshape(S, n)
+    dev = np.ascontiguousarray(is_device, dtype=np.uint8).reshape(S, n)
+    out = (NbDiag * S)()
+    secs = C.c_double(0)
+    _check(lib().nb_diagnostics(gpu, S, n, _d(q), _d(v), _d(m), _u(dev), step, out, C.byref(secs)))
+    res = [d.as_dict() for d in out]
+    res = res[0] if one else res
+    return (res, secs.value) if return_seconds else res
 
 
 def ensemble_run(q, v, m, is_device, planet, asteroid, kind=KIND_PLAIN, destroy_device=None, step_begin=0,

@@ -47,12 +47,14 @@ struct FstDev {
 };
 static FstDev g_fst_dev[64];
 
+double fst_at(int step) { return fabs(sin((step * NB_DT) / 6000)); }
+
 // grows the host table to at least min_len entries; call with g_fst_mu held
 static void fst_grow_locked(int min_len) {
     if ((int)g_fst_host.size() < min_len) {
         int len = min_len < NB_N_STEPS + 2 ? NB_N_STEPS + 2 : min_len;
         std::vector<double> t(len);
-        for (int s = 0; s < len; s++) t[s] = fabs(sin((s * NB_DT) / 6000));
+        for (int s = 0; s < len; s++) t[s] = fst_at(s);
         g_fst_host.swap(t);
     }
 }
@@ -550,6 +552,93 @@ int nb_traj_destroy(nb_traj* t) {
     t->b.release();
     delete t;
     return NB_OK;
+}
+
+// ---- diagnostics (nb_diag.cu) ---------------------------------------------------------------------------
+// [S][9] device results -> nb_diag
+static void diag_unpack(const double* r, int S, int n, int step, nb_diag* out) {
+    for (int s = 0; s < S; s++, r += 9) {
+        nb_diag& d = out[s];
+        d.step = step, d.n = n;
+        d.mass = r[0], d.kinetic = r[1], d.potential = r[2];
+        for (int c = 0; c < 3; c++) d.momentum[c] = r[3 + c], d.angular_momentum[c] = r[6 + c];
+    }
+}
+
+int nb_diagnostics(int gpu, int n_systems, int n, const double* q, const double* v, const double* m,
+                   const unsigned char* is_device, int step, nb_diag* out, double* gpu_seconds) {
+    if (n_systems < 1 || n < 1 || !q || !v || !m || !is_device || !out || step < 0) return NB_ERR_ARG;
+    int rc = nb::check_gpu(gpu);
+    if (rc) return rc;
+    NB_CUDA(cudaSetDevice(gpu));
+    const size_t S = (size_t)n_systems, qb = S * 3 * n * sizeof(double);
+    cudaStream_t st = nullptr;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    double *dq = nullptr, *dv = nullptr, *dm = nullptr, *dout = nullptr;
+    unsigned char* ddev = nullptr;
+    void* scratch = nullptr;
+    std::vector<double> res(S * 9);
+    auto chk = [&](cudaError_t e, const char* what) {
+        if (e != cudaSuccess && rc == NB_OK) rc = nb::cuda_fail(e, what, __FILE__, __LINE__);
+    };
+    chk(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking), "cudaStreamCreate");
+    chk(cudaEventCreate(&e0), "cudaEventCreate");
+    chk(cudaEventCreate(&e1), "cudaEventCreate");
+    chk(cudaMalloc(&dq, qb), "cudaMalloc q");
+    chk(cudaMalloc(&dv, qb), "cudaMalloc v");
+    chk(cudaMalloc(&dm, S * n * sizeof(double)), "cudaMalloc m");
+    chk(cudaMalloc(&ddev, S * n), "cudaMalloc is_device");
+    chk(cudaMalloc(&dout, S * 9 * sizeof(double)), "cudaMalloc out");
+    chk(cudaMalloc(&scratch, nb::diag_scratch_bytes(n_systems, n)), "cudaMalloc scratch");
+    if (rc == NB_OK) {
+        chk(cudaMemcpyAsync(dq, q, qb, cudaMemcpyHostToDevice, st), "H2D q");
+        chk(cudaMemcpyAsync(dv, v, qb, cudaMemcpyHostToDevice, st), "H2D v");
+        chk(cudaMemcpyAsync(dm, m, S * n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D m");
+        chk(cudaMemcpyAsync(ddev, is_device, S * n, cudaMemcpyHostToDevice, st), "H2D is_device");
+        chk(cudaEventRecord(e0, st), "cudaEventRecord");
+    }
+    if (rc == NB_OK) rc = nb::diag_launch(n_systems, n, dq, dv, dm, ddev, nb::fst_at(step), scratch, dout, st);
+    if (rc == NB_OK) {
+        chk(cudaEventRecord(e1, st), "cudaEventRecord");
+        chk(cudaMemcpyAsync(res.data(), dout, S * 9 * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H out");
+        chk(cudaStreamSynchronize(st), "sync");
+    }
+    if (rc == NB_OK) {
+        float ms = 0;
+        chk(cudaEventElapsedTime(&ms, e0, e1), "cudaEventElapsedTime");
+        if (gpu_seconds) *gpu_seconds = ms * 1e-3;
+        diag_unpack(res.data(), n_systems, n, step, out);
+    }
+    cudaFree(dq), cudaFree(dv), cudaFree(dm), cudaFree(ddev), cudaFree(dout), cudaFree(scratch);
+    if (e0) cudaEventDestroy(e0);
+    if (e1) cudaEventDestroy(e1);
+    if (st) cudaStreamDestroy(st);
+    return rc;
+}
+
+// slot 0 of the handle's batch, on its stream: q, v stay on the device
+int nb_traj_diagnostics(nb_traj* t, nb_diag* out) {
+    if (!t || !out) return NB_ERR_ARG;
+    DeviceBatch& b = t->b;
+    NB_CUDA(cudaSetDevice(b.gpu));
+    const int n = b.n, step = b.cur_step[0];
+    void* scratch = nullptr;
+    double* dout = nullptr;
+    double res[9];
+    int rc = NB_OK;
+    auto chk = [&](cudaError_t e, const char* what) {
+        if (e != cudaSuccess && rc == NB_OK) rc = nb::cuda_fail(e, what, __FILE__, __LINE__);
+    };
+    chk(cudaMalloc(&scratch, nb::diag_scratch_bytes(1, n)), "cudaMalloc scratch");
+    chk(cudaMalloc(&dout, 9 * sizeof(double)), "cudaMalloc out");
+    if (rc == NB_OK) rc = nb::diag_launch(1, n, b.q, b.v, b.m, b.isdev, nb::fst_at(step), scratch, dout, b.stream);
+    if (rc == NB_OK) {
+        chk(cudaMemcpyAsync(res, dout, sizeof res, cudaMemcpyDeviceToHost, b.stream), "D2H out");
+        chk(cudaStreamSynchronize(b.stream), "sync");
+    }
+    if (rc == NB_OK) diag_unpack(res, 1, n, step, out);
+    cudaFree(scratch), cudaFree(dout);
+    return rc;
 }
 
 // ---- ensembles ---------------------------------------------------------------------------------------

@@ -47,6 +47,15 @@ int sym_restart(nb_sym* h);
 int fst_table(int gpu, int min_len, const double** table_dev);
 double fst_value(int step);
 
+// nb_diag.cu: the diagnostics of S systems of n bodies (device arrays laid out as nb_diagnostics' host arrays) with the
+// masses of the step whose |sin| is fst; out = [S][9] doubles {mass, kinetic, potential, P[3], L[3]}.  Tile edge DIAG_T.
+constexpr int DIAG_T = 256;
+size_t diag_scratch_bytes(int S, int n);
+int diag_launch(int S, int n, const double* q, const double* v, const double* m, const unsigned char* is_device, double fst,
+                void* scratch, double* out, cudaStream_t stream);
+// |sin(step*dt/6000)| of any step >= 0, the expression the table is built with
+double fst_at(int step);
+
 // nb_traj.cu: n_traj single-block persistent trajectories of the same n in one launch
 int launch_traj_batch(int math, int n, int n_traj, const TrajDesc* descs_dev, const double* fst_dev,
                       cudaStream_t stream);

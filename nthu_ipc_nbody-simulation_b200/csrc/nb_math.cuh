@@ -32,12 +32,14 @@ __device__ __forceinline__ double rsqrt_seed(double x) {
     return y;
 }
 
-// G * m_eff of a body at a step: nbody.cc:14-16 with t = step*dt folded into fst = |sin(step*dt/6000)|
-// (host glibc table), then the first product of `G * mj * dx / dist3` (nbody.cc:70) hoisted.
+// m_eff of a body at a step: nbody.cc:14-16 with t = step*dt folded into fst = |sin(step*dt/6000)| (host glibc)
+__device__ __forceinline__ double m_eff(double m0, bool is_device, double fst) {
+    return is_device ? __dadd_rn(m0, __dmul_rn(__dmul_rn(0.5, m0), fst)) : m0;
+}
+
+// G * m_eff, the first product of `G * mj * dx / dist3` (nbody.cc:70) hoisted.
 __device__ __forceinline__ double gm_eff(double m0, bool is_device, double fst) {
-    double mj = m0;
-    if (is_device) mj = __dadd_rn(m0, __dmul_rn(__dmul_rn(0.5, m0), fst));
-    return __dmul_rn(G, mj);
+    return __dmul_rn(G, m_eff(m0, is_device, fst));
 }
 
 // d^2 between two bodies, evaluated exactly like nbody.cc:131-134 / hw5.cu:255-259 (no FMA), so
@@ -112,6 +114,17 @@ __device__ __forceinline__ void pair_sym(double xi, double yi, double zi, double
     ajx = fma(-cj, dx, ajx);
     ajy = fma(-cj, dy, ajy);
     ajz = fma(-cj, dz, ajz);
+}
+
+// FAST softened r^-1 of one pair (the potential, nb_diag.cu): r2 by pair_sym's FMA chain, eps^2 included,
+// y0 = rsqrt seed, e = 1 - r2*y0^2, r^-1 = y0*(1 + e/2 + 3e^2/8) (truncation ~ (5/16)|e|^3 < 2^-55 at the seed's
+// measured accuracy).  11 FP64-pipe instructions; the caller's accumulate FMA makes 12 per unordered pair.
+__device__ __forceinline__ double pair_rinv(double xi, double yi, double zi, double xj, double yj, double zj) {
+    const double dx = xj - xi, dy = yj - yi, dz = zj - zi;
+    const double r2 = fma(dx, dx, fma(dy, dy, fma(dz, dz, EPS2)));
+    const double y0 = rsqrt_seed(r2);
+    const double e = fma(-r2, y0 * y0, 1.0);
+    return fma(y0, e * fma(e, 0.375, 0.5), y0);
 }
 
 // v += a*dt; q += v*dt (nbody.cc:77-88, hw5.cu:235-236).  O(n) per step, so both math modes keep

@@ -8,6 +8,8 @@
 //                                                          (config C4), same n, split over all visible GPUs, one
 //                                                          line per member: k min_dist argmin_step hit_step
 //   nbtool ensemble-list <list.txt> <steps> <out.txt>      the same for the input files named in list.txt (equal n)
+//   nbtool diag <in> [step=0]                              mass, energies, momentum and angular momentum of the state
+//                                                          with the masses of `step` (nb_diagnostics), one line each
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -81,7 +83,8 @@ int usage() {
             "usage: nbtool gen <n> <seed> <out.in> [n_devices]\n"
             "       nbtool advance <in> <steps> <out.in>\n"
             "       nbtool ensemble <in> <members> <steps> <out.txt>\n"
-            "       nbtool ensemble-list <list.txt> <steps> <out.txt>\n");
+            "       nbtool ensemble-list <list.txt> <steps> <out.txt>\n"
+            "       nbtool diag <in> [step]\n");
     return 2;
 }
 
@@ -110,6 +113,23 @@ int main(int argc, char** argv) {
         if (rc) return fail(rc, "advance");
         rc = nb_write_input(argv[4], s.n, s.planet, s.asteroid, s.q.data(), s.v.data(), s.m.data(), s.dev.data());
         return rc ? fail(rc, argv[4]) : 0;
+    }
+    if (cmd == "diag" && (argc == 3 || argc == 4)) {
+        Sys s;
+        int rc = load(argv[2], s);
+        if (rc) return fail(rc, argv[2]);
+        const int step = argc == 4 ? atoi(argv[3]) : 0;
+        nb_diag d;
+        double secs = 0;
+        rc = nb_diagnostics(0, 1, s.n, s.q.data(), s.v.data(), s.m.data(), s.dev.data(), step, &d, &secs);
+        if (rc) return fail(rc, "diag");
+        printf("step %d\nn %d\nmass %.17g\nkinetic %.17g\npotential %.17g\nenergy %.17g\n", d.step, d.n, d.mass, d.kinetic,
+               d.potential, d.kinetic + d.potential);
+        const char* axis = "xyz";
+        for (int c = 0; c < 3; c++) printf("momentum_%c %.17g\n", axis[c], d.momentum[c]);
+        for (int c = 0; c < 3; c++) printf("angular_momentum_%c %.17g\n", axis[c], d.angular_momentum[c]);
+        fprintf(stderr, "nbtool: %d bodies: %.6f s of kernels\n", s.n, secs);
+        return 0;
     }
     if ((cmd == "ensemble" && argc == 6) || (cmd == "ensemble-list" && argc == 5)) {
         std::vector<Sys> members;
