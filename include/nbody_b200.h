@@ -43,6 +43,7 @@ extern "C" {
 
 #define NB_MAX_DEVICES 64
 #define NB_MAX_SMALL_N 1024 /* largest system the persistent (shared-memory resident) kernels take */
+#define NB_MAX_ENSEMBLE_N 65536 /* largest n of nb_ensemble_run: one system's partial-row scratch is 24*n^2/128 bytes */
 
 /* physics constants of nbody.cc:9-20 (read-only; exported for callers that need them) */
 #define NB_N_STEPS 200000
@@ -160,9 +161,12 @@ int nb_diagnostics(int gpu, int n_systems, int n, const double* q, const double*
 int nb_traj_diagnostics(nb_traj* t, nb_diag* out);
 
 /* ---- ensembles ------------------------------------------------------------------------------
- * n_systems independent systems of the same n in one launch, one thread block per system
- * (north-star (c): batches of synthetic systems).  Arrays are system-major: q[s][3*n] ...
- * planet/asteroid/destroy_device are per system.  q, v are updated in place; ev[s] filled.
+ * n_systems independent systems of the same n, 1 <= n <= NB_MAX_ENSEMBLE_N (north-star (c): batches of synthetic
+ * systems).  n <= NB_MAX_SMALL_N: one launch of a persistent kernel, one thread block per system.  Larger n: every step
+ * is three launches for a whole group of systems (pair kernel, integrate, observers; DESIGN.md 4.7), groups sized to a
+ * fixed scratch budget; n > NB_MAX_ENSEMBLE_N returns NB_ERR_UNSUPPORTED.  Arrays are system-major: q[s][3*n] ...
+ * planet/asteroid/destroy_device are per system.  q, v are updated in place and returned at ev[s].steps_done (a Q2/Q3
+ * member that hits stops at its hit step); ev[s] filled.  A system's result depends only on its own inputs and n.
  */
 int nb_ensemble_run(int gpu, int math, int kind, int n_systems, int n, double* q, double* v,
                     const double* m, const unsigned char* is_device, const int* planet,

@@ -367,7 +367,8 @@ def diagnostics(q, v, m, is_device, step=0, gpu=0, return_seconds=False):
 
 def ensemble_run(q, v, m, is_device, planet, asteroid, kind=KIND_PLAIN, destroy_device=None, step_begin=0,
                  step_end=1, gpu=0, math=MATH_FAST):
-    """S systems of the same n in one launch.  q, v: [S, 3n] (updated in place); m: [S, n];
+    """S systems of the same n, any n <= 65 536 (n <= 1024: one launch; larger n: one launch per kernel and step for the
+    whole batch).  q, v: [S, 3n] (updated in place); m: [S, n];
     is_device: [S, n] uint8; planet / asteroid / destroy_device: [S] int32.  Returns (events, gpu_seconds)."""
     S, n3 = q.shape
     n = n3 // 3

@@ -35,15 +35,6 @@ struct PairSys {
     const unsigned char* is_device;  // [S][n]
 };
 
-// tile k of the upper triangle (row-major over J, I <= J): k = J(J+1)/2 + I
-__device__ __forceinline__ void tile_of(int k, int& I, int& J) {
-    int a = (int)((sqrt(8.0 * (double)k + 1.0) - 1.0) * 0.5);
-    while ((long long)a * (a + 1) / 2 > k) a--;
-    while ((long long)(a + 1) * (a + 2) / 2 <= k) a++;
-    J = a;
-    I = k - (int)((long long)a * (a + 1) / 2);
-}
-
 template <bool DIAG>
 __device__ __forceinline__ void tile_pairs(const double4* rec, const double (&xi)[DIAG_IPT], const double (&yi)[DIAG_IPT],
                                            const double (&zi)[DIAG_IPT], double (&acc)[DIAG_IPT]) {

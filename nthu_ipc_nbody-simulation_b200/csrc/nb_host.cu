@@ -85,6 +85,10 @@ int fst_table(int gpu, int min_len, const double** out) {
     return NB_OK;
 }
 
+static int cuda_fail_or_ok(cudaError_t e, const char* what) {
+    return e == cudaSuccess ? NB_OK : cuda_fail(e, what, __FILE__, __LINE__);
+}
+
 static int check_gpu(int gpu) {
     int cnt = 0;
     cudaError_t e = cudaGetDeviceCount(&cnt);
@@ -172,6 +176,10 @@ static int large_chunk(int n) {
     return (int)std::min(512LL, std::max(4LL, c));
 }
 
+// Ensembles of n > NB_MAX_SMALL_N (DeviceBatch::run_ens_large): the scratch of one group of systems stepped together (slots
+// and double-buffered records, nb_ens.cu) stays within this budget; the groups run one after another.
+constexpr size_t ENS_GROUP_BYTES = (size_t)2 << 30;
+
 // ---- a batch of same-n systems resident on one GPU ---------------------------------------------------
 struct DeviceBatch {
     int gpu = -1, S = 0, n = 0, math = 0;
@@ -192,13 +200,15 @@ struct DeviceBatch {
     double gpu_seconds = 0.0;
     long long pairs = 0;
     // n > NB_MAX_SMALL_N: the steppers, shared by the systems (they are stepped in turn), and the events of the system being
-    // stepped after each of the last two chunks (pinned staging, see run_large)
+    // stepped after each of the last two chunks (pinned staging, see run_large).  An ensemble (ens) has no stepper: its
+    // systems go in groups through nb_ens.cu (run_ens_large), and pin_chunk holds the events of a whole group twice.
     LargeStepper large;
+    bool ens = false;
     nb_events* pin_chunk = nullptr;
     cudaEvent_t chunk_done[2] = {nullptr, nullptr};
 
-    int init(int gpu_, int S_, int n_, int math_) {
-        gpu = gpu_, S = S_, n = n_, math = math_;
+    int init(int gpu_, int S_, int n_, int math_, bool ens_ = false) {
+        gpu = gpu_, S = S_, n = n_, math = math_, ens = ens_;
         NB_CUDA(cudaSetDevice(gpu));
         NB_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
         NB_CUDA(cudaEventCreate(&e0));
@@ -216,9 +226,11 @@ struct DeviceBatch {
         h_ev.assign(S, nb_events{});
         cur_step.assign(S, 0);
         if (n > NB_MAX_SMALL_N) {
-            const int rc = large.init(n, math, stream);
-            if (rc) return rc;
-            NB_CUDA(cudaHostAlloc(&pin_chunk, 2 * sizeof(nb_events), cudaHostAllocDefault));
+            if (!ens) {
+                const int rc = large.init(n, math, stream);
+                if (rc) return rc;
+            }
+            NB_CUDA(cudaHostAlloc(&pin_chunk, 2 * (size_t)(ens ? S : 1) * sizeof(nb_events), cudaHostAllocDefault));
             NB_CUDA(cudaEventCreateWithFlags(&chunk_done[0], cudaEventDisableTiming));
             NB_CUDA(cudaEventCreateWithFlags(&chunk_done[1], cudaEventDisableTiming));
         }
@@ -310,7 +322,7 @@ struct DeviceBatch {
         // ascending-j sum
         bool grid = false;
         if (n > NB_MAX_SMALL_N) {
-            rc = run_large();
+            rc = ens ? run_ens_large() : run_large();
         } else if (allow_grid && math == NB_MATH_FAST && max_dev <= 64 && grid_traj_supported(gpu, n)) {
             size_t need = grid_traj_workspace_bytes(n);
             if (need > grid_ws_bytes) {
@@ -392,6 +404,64 @@ struct DeviceBatch {
             if (rc) return rc;
         }
         return NB_OK;
+    }
+    // Ensembles of n > NB_MAX_SMALL_N: every system starts at the same step.  The systems go in groups of G whose scratch fits
+    // ENS_GROUP_BYTES; a group is packed (one nb_large_pack per system), its step_begin observed unless it already was, and
+    // stepped by three launches per step for all its systems (ens_step, ens_observe).  Steps go out in chunks as in
+    // run_large; the host reads the group's events after each chunk and enqueues nothing more once every member has stopped.
+    // A stopped member returns at the top of every kernel, so its records and v stay at its hit step, and each member is
+    // unpacked from the records of its own steps_done.
+    int run_ens_large() {
+        const int n_pad = ens_pad(n), n_slots = ens_slots(math, n);
+        const size_t per_sys = ((size_t)n_slots * 3 * sizeof(double) + 2 * sizeof(double4)) * n_pad;
+        const int G_max = (int)std::max<size_t>(1, std::min<size_t>({(size_t)S, ENS_GROUP_BYTES / per_sys, 65535}));
+        const int step0 = h_descs[0].step_begin, step_end = h_descs[0].step_end;
+        double4* pos4 = nullptr;
+        double* slots = nullptr;
+        NB_CUDA(cudaMalloc(&pos4, 2 * (size_t)G_max * n_pad * sizeof(double4)));
+        int rc = cuda_fail_or_ok(cudaMalloc(&slots, (size_t)G_max * n_slots * 3 * n_pad * sizeof(double)), "cudaMalloc slots");
+        // the records past n are zero (massless, at the origin) for good: nothing writes them
+        if (!rc) rc = cuda_fail_or_ok(cudaMemsetAsync(pos4, 0, 2 * (size_t)G_max * n_pad * sizeof(double4), stream), "memset");
+        for (int s0 = 0; s0 < S && !rc; s0 += G_max) {
+            const EnsGroup e{descs + s0, pos4, slots, n, n_pad, n_slots, std::min(G_max, S - s0)};
+            const long long work = (long long)e.G * n * n;
+            const int chunk = (int)std::min(512LL, std::max(4LL, (1LL << 33) / work));
+            for (int g = 0; g < e.G && !rc; g++) {
+                const TrajDesc& d = h_descs[s0 + g];
+                double* rec = (double*)(pos4 + ((size_t)(step0 & 1) * e.G + g) * n_pad);
+                rc = nb_large_pack(math, n, d.q, d.m, d.is_device, step0 + 1, rec, stream);
+            }
+            if (!rc) rc = ens_observe(e, step0, stream);
+            for (int st = step0, c = 0; !rc && st < step_end; c++) {
+                const int end = std::min(st + chunk, step_end);
+                while (!rc && st < end) {
+                    rc = ens_step(math, e, ++st, stream);
+                    if (!rc) rc = ens_observe(e, st, stream);
+                }
+                if (rc || st >= step_end) break;
+                nb_events* pin = pin_chunk + (size_t)(c & 1) * S;
+                rc = cuda_fail_or_ok(cudaMemcpyAsync(pin, ev + s0, e.G * sizeof(nb_events), cudaMemcpyDeviceToHost, stream),
+                                     "D2H chunk events");
+                if (!rc) rc = cuda_fail_or_ok(cudaEventRecord(chunk_done[c & 1], stream), "cudaEventRecord");
+                if (!rc && c > 0) {  // chunk c is queued: read the events after chunk c - 1
+                    rc = spin_wait(stream, chunk_done[(c - 1) & 1]);
+                    const nb_events* prev = pin_chunk + (size_t)((c - 1) & 1) * S;
+                    bool all = true;
+                    for (int g = 0; g < e.G && all; g++) all = stopped(prev[g], h_descs[s0 + g].kind);
+                    if (!rc && all) break;
+                }
+            }
+            // each member's records of its own last step
+            if (!rc) rc = cuda_fail_or_ok(cudaMemcpyAsync(pin_chunk, ev + s0, e.G * sizeof(nb_events), cudaMemcpyDeviceToHost,
+                                                          stream), "D2H group events");
+            if (!rc) rc = spin_wait(stream);
+            for (int g = 0; g < e.G && !rc; g++)
+                rc = nb_large_unpack(n, (const double*)(pos4 + ((size_t)(pin_chunk[g].steps_done & 1) * e.G + g) * n_pad),
+                                     h_descs[s0 + g].q, stream);
+        }
+        if (!rc) rc = spin_wait(stream);
+        cudaFree(pos4), cudaFree(slots);
+        return rc;
     }
     int get_state(int s, double* hq, double* hv, double* hm) {
         NB_CUDA(cudaSetDevice(gpu));
@@ -646,13 +716,13 @@ int nb_ensemble_run(int gpu, int math, int kind, int n_systems, int n, double* q
                     const unsigned char* is_device, const int* planet, const int* asteroid, const int* destroy_device,
                     int step_begin, int step_end, nb_events* ev, double* gpu_seconds) {
     if (n_systems < 1 || n < 1 || !q || !v || !m || !is_device || step_begin < 0 || step_end < step_begin) return NB_ERR_ARG;
-    if (n > NB_MAX_SMALL_N) return NB_ERR_UNSUPPORTED;
+    if (n > NB_MAX_ENSEMBLE_N) return NB_ERR_UNSUPPORTED;
     if (kind < NB_KIND_PLAIN || kind > NB_KIND_Q3 || (math != NB_MATH_FAST && math != NB_MATH_STRICT)) return NB_ERR_ARG;
     if (kind == NB_KIND_Q3 && !destroy_device) return NB_ERR_ARG;
     int rc = nb::check_gpu(gpu);
     if (rc) return rc;
     DeviceBatch b;
-    rc = b.init(gpu, n_systems, n, math);
+    rc = b.init(gpu, n_systems, n, math, true);
     for (int s = 0; s < n_systems && !rc; s++)
         rc = b.set_system(s, q + (size_t)s * 3 * n, v + (size_t)s * 3 * n, m + (size_t)s * n, is_device + (size_t)s * n,
                           planet ? planet[s] : 0, asteroid ? asteroid[s] : 0, kind,

@@ -56,6 +56,21 @@ int diag_launch(int S, int n, const double* q, const double* v, const double* m,
 // |sin(step*dt/6000)| of any step >= 0, the expression the table is built with
 double fst_at(int step);
 
+// nb_ens.cu: ensembles of n > NB_MAX_SMALL_N bodies, G systems stepped by one launch per kernel.  A system's records are
+// pos4 + (parity * G + g) * n_pad (parity = step & 1), its partial accelerations slots + g * n_slots * 3 * n_pad.
+struct EnsGroup {
+    const TrajDesc* descs;  // [G] device
+    double4* pos4;          // [2][G][n_pad] {x, y, z, G*m_eff}; bodies n .. n_pad-1 zero
+    double* slots;          // [G][n_slots][3][n_pad]
+    int n, n_pad, n_slots, G;
+};
+int ens_pad(int n);              // bodies per system record buffer: whole tiles
+int ens_slots(int math, int n);  // partial-acceleration slots per body
+// step `step` (reads the records of step - 1, writes those of step): the pair kernel and the integrate kernel
+int ens_step(int math, const EnsGroup& e, int step, cudaStream_t stream);
+// the observers of step `step` on its records, one warp per system
+int ens_observe(const EnsGroup& e, int step, cudaStream_t stream);
+
 // nb_traj.cu: n_traj single-block persistent trajectories of the same n in one launch
 int launch_traj_batch(int math, int n, int n_traj, const TrajDesc* descs_dev, const double* fst_dev,
                       cudaStream_t stream);

@@ -127,6 +127,15 @@ __device__ __forceinline__ double pair_rinv(double xi, double yi, double zi, dou
     return fma(y0, e * fma(e, 0.375, 0.5), y0);
 }
 
+// tile k of the upper triangle of a tiled pair matrix (row-major over J, I <= J): k = J(J+1)/2 + I.  nb_diag.cu, nb_ens.cu
+__device__ __forceinline__ void tile_of(int k, int& I, int& J) {
+    int a = (int)((sqrt(8.0 * (double)k + 1.0) - 1.0) * 0.5);
+    while ((long long)a * (a + 1) / 2 > k) a--;
+    while ((long long)(a + 1) * (a + 2) / 2 <= k) a++;
+    J = a;
+    I = k - (int)((long long)a * (a + 1) / 2);
+}
+
 // v += a*dt; q += v*dt (nbody.cc:77-88, hw5.cu:235-236).  O(n) per step, so both math modes keep
 // the reference's four separate roundings (no FMA): the state update is then exactly run_step's.
 __device__ __forceinline__ void kick_drift(double a, double& v, double& q) {

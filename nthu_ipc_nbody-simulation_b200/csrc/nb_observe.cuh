@@ -1,6 +1,6 @@
 // The in-kernel observers of one trajectory, shared by traj_kernel, traj_sym_kernel (nb_traj.cu), the observer warp of
-// grid_traj_kernel (nb_grid.cu) and large_observe_kernel (nb_large.cu, n > 1024): minimum distance, missile reach, hit test and the Q3 destroy (hw5.cu:241-309), and the
-// gravity devices' mass rule.  Every comparison is the reference's un-contracted arithmetic (dist2_rn), so the discrete
+// grid_traj_kernel (nb_grid.cu) and the large-N observers (observe_large, n > 1024): minimum distance, missile reach, hit
+// test and the Q3 destroy (hw5.cu:241-309), and the gravity devices' mass rule.  Every comparison is the reference's un-contracted arithmetic (dist2_rn), so the discrete
 // outputs do not depend on the math mode.
 #pragma once
 #include "nb_internal.h"
@@ -93,6 +93,41 @@ __device__ __forceinline__ int observe_step(Observed& ob, int st, int kind, int 
         }
     }
     return 0;
+}
+
+// The observers of step st of one trajectory on the large-N steppers (large_observe_kernel, large_ens_observe_kernel): one
+// warp reads the records {x, y, z, G*m_eff(st+1)} the step's integrate kernel wrote.  Lane l looks after devices l and
+// l + 32 (NB_MAX_DEVICES = 64), as the grid kernel's observer warp does.  A stopped trajectory (Q2/Q3 hit) or an already observed step is left as it is,
+// so steps enqueued past the stop change no event.  The Q3 destroy at st zeroes the device's base mass (Observed::store)
+// and the mass of the record just read: the forces of step st+1 are the first without it (hw5.cu:299-307).
+__device__ __forceinline__ void observe_large(const TrajDesc& d, double4* __restrict__ pos4, int st) {
+    const int lane = threadIdx.x;
+    Observed ob;
+    ob.load(d.ev);
+    const bool stopped = (d.kind >= NB_KIND_Q2) && ob.hit_step != -2;
+    if (stopped || d.ev->steps_done >= st) return;
+    int my_dev[2], my_reach[2];
+#pragma unroll
+    for (int h = 0; h < 2; h++) {
+        const int k = lane + 32 * h;
+        my_dev[h] = k < d.n_dev ? d.dev_index[k] : -1;
+        my_reach[h] = k < d.n_dev ? d.ev->reach_step[k] : -2;
+    }
+    const int DD = d.destroy_device;
+    const bool armed = q3_armed(d.kind, DD, d.n, d.m);
+    const int seen = observe_step<2>(ob, st, d.kind, d.planet, d.asteroid, armed, armed ? DD : 0, my_dev, my_reach,
+                                     [&](int r, double& x, double& y, double& z) {
+                                         const double4 p = pos4[r];
+                                         x = p.x, y = p.y, z = p.z;
+                                     });
+    __syncwarp();  // every lane has read the events before lane 0 rewrites them
+#pragma unroll
+    for (int h = 0; h < 2; h++)
+        if (lane + 32 * h < d.n_dev) d.ev->reach_step[lane + 32 * h] = my_reach[h];
+    if (lane == 0) {
+        ob.store(d, st);
+        if (seen == OBS_DESTROYED) pos4[DD].w = 0.0;
+    }
 }
 
 }  // namespace nb
