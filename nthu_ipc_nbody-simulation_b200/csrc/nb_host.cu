@@ -29,8 +29,6 @@ int cuda_fail(cudaError_t e, const char* what, const char* file, int line) {
     return NB_ERR_CUDA;
 }
 static std::atomic<long long> g_launches{0};
-// set by nb_hw5_main: the process leaves through _exit right after the output file is written, so device buffers,
-// pinned mailboxes and streams are not torn down one by one (cudaFree / cudaFreeHost cost up to 0.7 s there)
 std::atomic<bool> g_leak_on_exit{false};
 static std::atomic<long long> g_torn_records{0};
 void count_launch(int n) { g_launches += n; }
@@ -85,10 +83,6 @@ int fst_table(int gpu, int min_len, const double** out) {
     return NB_OK;
 }
 
-static int cuda_fail_or_ok(cudaError_t e, const char* what) {
-    return e == cudaSuccess ? NB_OK : cuda_fail(e, what, __FILE__, __LINE__);
-}
-
 static int check_gpu(int gpu) {
     int cnt = 0;
     cudaError_t e = cudaGetDeviceCount(&cnt);
@@ -126,55 +120,44 @@ static int spin_wait(cudaStream_t stream, cudaEvent_t e = nullptr) {
 // planar [3][n] and its v is stepped in place.  Used by nb_run_steps and by the query path (DeviceBatch::run).
 struct LargeStepper {
     int n = 0, math = 0, cur = 0;  // pos[cur] holds the current step
-    nb_sym* h = nullptr;
-    double* pos[2] = {nullptr, nullptr};
-    void* work = nullptr;
+    SymHandle h;
+    DeviceMem<double> pos[2];
+    DeviceMem<void> work;
 
     // on the current device; the PJ zero-fill is enqueued on st
     int init(int n_, int math_, cudaStream_t st) {
         n = n_, math = math_;
         if (math == NB_MATH_FAST) {
-            const int rc = nb_sym_create(n, 1, 0, &h);
+            nb_sym* raw = nullptr;
+            const int rc = nb_sym_create(n, 1, 0, &raw);
             if (rc) return rc;
+            h.reset(raw);
         }
-        NB_CUDA(cudaMalloc(&pos[0], 4 * (size_t)n * sizeof(double)));
-        NB_CUDA(cudaMalloc(&pos[1], 4 * (size_t)n * sizeof(double)));
-        const size_t bytes = (size_t)(h ? nb_sym_pj_bytes(h) : nb_large_scratch_bytes(n, n));
-        NB_CUDA(cudaMalloc(&work, bytes));
-        if (h) NB_CUDA(cudaMemsetAsync(work, 0, bytes, st));  // PJ rows nobody writes are summed as zeros
+        NB_CUDA(alloc(pos[0], 4 * (size_t)n * sizeof(double)));
+        NB_CUDA(alloc(pos[1], 4 * (size_t)n * sizeof(double)));
+        const size_t bytes = (size_t)(h ? nb_sym_pj_bytes(h.get()) : nb_large_scratch_bytes(n, n));
+        NB_CUDA(alloc(work, bytes));
+        if (h) NB_CUDA(cudaMemsetAsync(work.get(), 0, bytes, st));  // PJ rows nobody writes are summed as zeros
         return NB_OK;
     }
     // planar positions of step step_next - 1 with the masses of step_next: the next step() is step_next, any step
     int pack(const double* q, const double* m, const unsigned char* is_device, int step_next, cudaStream_t st) {
         cur = 0;
         if (h) {
-            const int rc = sym_restart(h);
+            const int rc = sym_restart(h.get());
             if (rc) return rc;
         }
-        return nb_large_pack(math, n, q, m, is_device, step_next, pos[0], st);
+        return nb_large_pack(math, n, q, m, is_device, step_next, pos[0].get(), st);
     }
     int step(int s, double* v, const double* m, const unsigned char* is_device, cudaStream_t st) {
-        double *next = pos[cur ^ 1], *pj = (double*)work;
-        const int rc = h ? nb_sym_step(h, s, pos[cur], &next, &pj, nullptr, nullptr, v, m, is_device, st)
-                         : nb_large_step(math, s, n, 0, n, pos[cur], next, v, m, is_device, work, st);
+        double *next = pos[cur ^ 1].get(), *pj = (double*)work.get();
+        const int rc = h ? nb_sym_step(h.get(), s, pos[cur].get(), &next, &pj, nullptr, nullptr, v, m, is_device, st)
+                         : nb_large_step(math, s, n, 0, n, pos[cur].get(), next, v, m, is_device, work.get(), st);
         if (!rc) cur ^= 1;
         return rc;
     }
-    int unpack(double* q, cudaStream_t st) { return nb_large_unpack(n, pos[cur], q, st); }
-    void release() {
-        cudaFree(pos[0]), cudaFree(pos[1]), cudaFree(work);
-        if (h) nb_sym_destroy(h);
-        *this = LargeStepper{};
-    }
+    int unpack(double* q, cudaStream_t st) { return nb_large_unpack(n, pos[cur].get(), q, st); }
 };
-
-// Steps per chunk of the query path on the large-N steppers: the host reads the events between chunks.  A step costs
-// about n^2 (2.95 ms at 65 536 bodies on the B200), so 2^33 / n^2 steps, at least 4 (~12 ms at 65 536 bodies) and at most
-// 512 (below ~4 096 bodies a step is bound by launch latency).
-static int large_chunk(int n) {
-    const long long c = (1LL << 33) / ((long long)n * n);
-    return (int)std::min(512LL, std::max(4LL, c));
-}
 
 // Ensembles of n > NB_MAX_SMALL_N (DeviceBatch::run_ens_large): the scratch of one group of systems stepped together (slots
 // and double-buffered records, nb_ens.cu) stays within this budget; the groups run one after another.
@@ -183,80 +166,62 @@ constexpr size_t ENS_GROUP_BYTES = (size_t)2 << 30;
 // ---- a batch of same-n systems resident on one GPU ---------------------------------------------------
 struct DeviceBatch {
     int gpu = -1, S = 0, n = 0, math = 0;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    double *q = nullptr, *v = nullptr, *m = nullptr;
-    unsigned char* isdev = nullptr;
-    int* devidx = nullptr;
-    nb_events* ev = nullptr;
-    TrajDesc* descs = nullptr;
-    void* grid_ws = nullptr;
+    Stream stream;
+    Event e0, e1;
+    DeviceMem<double> q, v, m;
+    DeviceMem<unsigned char> isdev;
+    DeviceMem<int> devidx;
+    DeviceMem<nb_events> ev;
+    DeviceMem<TrajDesc> descs;
+    DeviceMem<void> grid_ws;
     size_t grid_ws_bytes = 0;
     std::vector<TrajDesc> h_descs;
     std::vector<nb_events> h_ev;
-    nb_events* pin_ev = nullptr;  // pinned staging for the events + the grid kernel's status word: the D2H copies after a
-    int* pin_status = nullptr;    // launch are then truly asynchronous and run() does the waiting itself (busy-wait)
+    PinnedMem<nb_events> pin_ev;  // pinned staging for the events + the grid kernel's status word: the D2H copies after a
+    PinnedMem<int> pin_status;    // launch are then truly asynchronous and run() does the waiting itself (busy-wait)
     std::vector<int> cur_step;
     double gpu_seconds = 0.0;
     long long pairs = 0;
-    // n > NB_MAX_SMALL_N: the steppers, shared by the systems (they are stepped in turn), and the events of the system being
-    // stepped after each of the last two chunks (pinned staging, see run_large).  An ensemble (ens) has no stepper: its
-    // systems go in groups through nb_ens.cu (run_ens_large), and pin_chunk holds the events of a whole group twice.
+    // n > NB_MAX_SMALL_N: the steppers, shared by the systems (they are stepped in turn), and the events of the systems
+    // being stepped after each of the last two chunks (pinned staging, see run_chunks).  An ensemble (ens) has no stepper:
+    // its systems go in groups through nb_ens.cu (run_ens_large), and pin_chunk holds the events of a whole group twice.
     LargeStepper large;
     bool ens = false;
-    nb_events* pin_chunk = nullptr;
-    cudaEvent_t chunk_done[2] = {nullptr, nullptr};
+    PinnedMem<nb_events> pin_chunk;
+    Event chunk_done[2];
 
+    // the members are freed after this body, on the batch's GPU (nb_solve runs one host thread per GPU)
+    ~DeviceBatch() {
+        if (gpu >= 0) cudaSetDevice(gpu);
+    }
     int init(int gpu_, int S_, int n_, int math_, bool ens_ = false) {
         gpu = gpu_, S = S_, n = n_, math = math_, ens = ens_;
         NB_CUDA(cudaSetDevice(gpu));
-        NB_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-        NB_CUDA(cudaEventCreate(&e0));
-        NB_CUDA(cudaEventCreate(&e1));
-        NB_CUDA(cudaMalloc(&q, (size_t)S * 3 * n * sizeof(double)));
-        NB_CUDA(cudaMalloc(&v, (size_t)S * 3 * n * sizeof(double)));
-        NB_CUDA(cudaMalloc(&m, (size_t)S * n * sizeof(double)));
-        NB_CUDA(cudaMalloc(&isdev, (size_t)S * n));
-        NB_CUDA(cudaMalloc(&devidx, (size_t)S * NB_MAX_DEVICES * sizeof(int)));
-        NB_CUDA(cudaMalloc(&ev, (size_t)S * sizeof(nb_events)));
-        NB_CUDA(cudaMalloc(&descs, (size_t)S * sizeof(TrajDesc)));
-        NB_CUDA(cudaHostAlloc(&pin_ev, (size_t)S * sizeof(nb_events), cudaHostAllocDefault));
-        NB_CUDA(cudaHostAlloc(&pin_status, 64, cudaHostAllocDefault));
+        NB_CUDA(create(stream));
+        NB_CUDA(create(e0));
+        NB_CUDA(create(e1));
+        NB_CUDA(alloc(q, (size_t)S * 3 * n * sizeof(double)));
+        NB_CUDA(alloc(v, (size_t)S * 3 * n * sizeof(double)));
+        NB_CUDA(alloc(m, (size_t)S * n * sizeof(double)));
+        NB_CUDA(alloc(isdev, (size_t)S * n));
+        NB_CUDA(alloc(devidx, (size_t)S * NB_MAX_DEVICES * sizeof(int)));
+        NB_CUDA(alloc(ev, (size_t)S * sizeof(nb_events)));
+        NB_CUDA(alloc(descs, (size_t)S * sizeof(TrajDesc)));
+        NB_CUDA(alloc(pin_ev, (size_t)S * sizeof(nb_events)));
+        NB_CUDA(alloc(pin_status, 64));
         h_descs.assign(S, TrajDesc{});
         h_ev.assign(S, nb_events{});
         cur_step.assign(S, 0);
         if (n > NB_MAX_SMALL_N) {
             if (!ens) {
-                const int rc = large.init(n, math, stream);
+                const int rc = large.init(n, math, stream.get());
                 if (rc) return rc;
             }
-            NB_CUDA(cudaHostAlloc(&pin_chunk, 2 * (size_t)(ens ? S : 1) * sizeof(nb_events), cudaHostAllocDefault));
-            NB_CUDA(cudaEventCreateWithFlags(&chunk_done[0], cudaEventDisableTiming));
-            NB_CUDA(cudaEventCreateWithFlags(&chunk_done[1], cudaEventDisableTiming));
+            NB_CUDA(alloc(pin_chunk, 2 * (size_t)(ens ? S : 1) * sizeof(nb_events)));
+            NB_CUDA(create(chunk_done[0], cudaEventDisableTiming));
+            NB_CUDA(create(chunk_done[1], cudaEventDisableTiming));
         }
         return NB_OK;
-    }
-    void release() {
-        if (gpu < 0) return;
-        if (g_leak_on_exit.load()) {
-            gpu = -1;
-            return;
-        }
-        cudaSetDevice(gpu);
-        cudaFree(q), cudaFree(v), cudaFree(m), cudaFree(isdev), cudaFree(devidx), cudaFree(ev), cudaFree(descs);
-        if (grid_ws) cudaFree(grid_ws);
-        if (pin_ev) cudaFreeHost(pin_ev);
-        if (pin_status) cudaFreeHost(pin_status);
-        pin_ev = nullptr, pin_status = nullptr;
-        large.release();
-        if (pin_chunk) cudaFreeHost(pin_chunk);
-        pin_chunk = nullptr;
-        for (cudaEvent_t& e : chunk_done)
-            if (e) cudaEventDestroy(e), e = nullptr;
-        if (e0) cudaEventDestroy(e0);
-        if (e1) cudaEventDestroy(e1);
-        if (stream) cudaStreamDestroy(stream);
-        gpu = -1;
     }
     static void fresh_events(nb_events& e) {
         e.min_d2 = std::numeric_limits<double>::infinity();
@@ -282,23 +247,24 @@ struct DeviceBatch {
             }
         if ((int)di.size() > NB_MAX_DEVICES) return NB_ERR_UNSUPPORTED;
         NB_CUDA(cudaSetDevice(gpu));
+        double *sq = q.get() + (size_t)s * 3 * n, *sv = v.get() + (size_t)s * 3 * n, *sm = m.get() + (size_t)s * n;
+        unsigned char* sdev = isdev.get() + (size_t)s * n;
+        int* sidx = devidx.get() + (size_t)s * NB_MAX_DEVICES;
         // hq / hv may be null: the caller fills q, v device-to-device afterwards (nb_traj_fork)
-        if (hq) NB_CUDA(cudaMemcpyAsync(q + (size_t)s * 3 * n, hq, 3 * n * sizeof(double), cudaMemcpyHostToDevice, stream));
-        if (hv) NB_CUDA(cudaMemcpyAsync(v + (size_t)s * 3 * n, hv, 3 * n * sizeof(double), cudaMemcpyHostToDevice, stream));
-        NB_CUDA(cudaMemcpyAsync(m + (size_t)s * n, mm.data(), n * sizeof(double), cudaMemcpyHostToDevice, stream));
-        NB_CUDA(cudaMemcpyAsync(isdev + (size_t)s * n, hdev, n, cudaMemcpyHostToDevice, stream));
+        if (hq) NB_CUDA(cudaMemcpyAsync(sq, hq, 3 * n * sizeof(double), cudaMemcpyHostToDevice, stream.get()));
+        if (hv) NB_CUDA(cudaMemcpyAsync(sv, hv, 3 * n * sizeof(double), cudaMemcpyHostToDevice, stream.get()));
+        NB_CUDA(cudaMemcpyAsync(sm, mm.data(), n * sizeof(double), cudaMemcpyHostToDevice, stream.get()));
+        NB_CUDA(cudaMemcpyAsync(sdev, hdev, n, cudaMemcpyHostToDevice, stream.get()));
         if (!di.empty())
-            NB_CUDA(cudaMemcpyAsync(devidx + (size_t)s * NB_MAX_DEVICES, di.data(), di.size() * sizeof(int),
-                                    cudaMemcpyHostToDevice, stream));
+            NB_CUDA(cudaMemcpyAsync(sidx, di.data(), di.size() * sizeof(int), cudaMemcpyHostToDevice, stream.get()));
         fresh_events(h_ev[s]);
         h_ev[s].n_reach = (int)di.size();
-        NB_CUDA(cudaMemcpyAsync(ev + s, &h_ev[s], sizeof(nb_events), cudaMemcpyHostToDevice, stream));
-        NB_CUDA(cudaStreamSynchronize(stream));  // mm / di are stack-local
+        NB_CUDA(cudaMemcpyAsync(ev.get() + s, &h_ev[s], sizeof(nb_events), cudaMemcpyHostToDevice, stream.get()));
+        NB_CUDA(cudaStreamSynchronize(stream.get()));  // mm / di are stack-local
         TrajDesc& d = h_descs[s];
         d.n = n, d.planet = planet, d.asteroid = asteroid, d.kind = kind, d.destroy_device = destroy_device;
         d.n_dev = (int)di.size();
-        d.q = q + (size_t)s * 3 * n, d.v = v + (size_t)s * 3 * n, d.m = m + (size_t)s * n;
-        d.is_device = isdev + (size_t)s * n, d.dev_index = devidx + (size_t)s * NB_MAX_DEVICES, d.ev = ev + s;
+        d.q = sq, d.v = sv, d.m = sm, d.is_device = sdev, d.dev_index = sidx, d.ev = ev.get() + s;
         cur_step[s] = step0;
         return NB_OK;
     }
@@ -313,8 +279,8 @@ struct DeviceBatch {
         int rc = fst_table(gpu, max_end + 2, &fst);
         if (rc) return rc;
         NB_CUDA(cudaSetDevice(gpu));
-        NB_CUDA(cudaMemcpyAsync(descs, h_descs.data(), S * sizeof(TrajDesc), cudaMemcpyHostToDevice, stream));
-        NB_CUDA(cudaEventRecord(e0, stream));
+        NB_CUDA(cudaMemcpyAsync(descs.get(), h_descs.data(), S * sizeof(TrajDesc), cudaMemcpyHostToDevice, stream.get()));
+        NB_CUDA(cudaEventRecord(e0.get(), stream.get()));
         const auto h0 = std::chrono::steady_clock::now();
         int max_dev = 0;
         for (int s = 0; s < S; s++) max_dev = h_descs[s].n_dev > max_dev ? h_descs[s].n_dev : max_dev;
@@ -326,44 +292,47 @@ struct DeviceBatch {
         } else if (allow_grid && math == NB_MATH_FAST && max_dev <= 64 && grid_traj_supported(gpu, n)) {
             size_t need = grid_traj_workspace_bytes(n);
             if (need > grid_ws_bytes) {
-                if (grid_ws) NB_CUDA(cudaFree(grid_ws));
-                NB_CUDA(cudaMalloc(&grid_ws, need));
+                grid_ws.reset();  // the old workspace goes first: the new one may not fit beside it
+                NB_CUDA(alloc(grid_ws, need));
                 grid_ws_bytes = need;
             }
-            rc = launch_grid_traj(math, n, S, descs, fst, gpu, grid_ws, grid_ws_bytes, stream);
+            rc = launch_grid_traj(math, n, S, descs.get(), fst, gpu, grid_ws.get(), grid_ws_bytes, stream.get());
             grid = true;
             if (rc == NB_ERR_UNSUPPORTED) {
                 // the grid's blocks cannot be co-resident here (MIG, MPS, a shared GPU); nothing was launched and no
                 // state was touched: the single-block kernel gives the same answer, only slower
                 static const bool verbose = getenv("NB_VERBOSE") != nullptr;
                 if (verbose) fprintf(stderr, "nbody_b200: grid kernel unavailable (%s): single-block kernel instead\n", g_detail.c_str());
-                rc = launch_traj_batch(math, n, S, descs, fst, stream);
+                rc = launch_traj_batch(math, n, S, descs.get(), fst, stream.get());
                 grid = false;
             }
         } else {
-            rc = launch_traj_batch(math, n, S, descs, fst, stream);
+            rc = launch_traj_batch(math, n, S, descs.get(), fst, stream.get());
         }
         if (rc) return rc;
-        NB_CUDA(cudaEventRecord(e1, stream));  // e0 .. e1 = the kernels only: nothing below waits on the host in between
+        NB_CUDA(cudaEventRecord(e1.get(), stream.get()));  // e0 .. e1 = the kernels only: nothing below waits on the host in between
         {
             const double hms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - h0).count();
             static const bool verbose = getenv("NB_VERBOSE") != nullptr;
             if (verbose && hms > 2.0) fprintf(stderr, "nbody_b200:   host spent %.1f ms between the two event records\n", hms);
         }
-        NB_CUDA(cudaMemcpyAsync(pin_ev, ev, S * sizeof(nb_events), cudaMemcpyDeviceToHost, stream));
-        *pin_status = 0;
-        pin_status[1] = 0;
-        if (grid) NB_CUDA(cudaMemcpyAsync(pin_status, grid_traj_status(grid_ws, n), 2 * sizeof(int), cudaMemcpyDeviceToHost, stream));
-        rc = spin_wait(stream);
+        int* status = pin_status.get();
+        NB_CUDA(cudaMemcpyAsync(pin_ev.get(), ev.get(), S * sizeof(nb_events), cudaMemcpyDeviceToHost, stream.get()));
+        status[0] = 0;
+        status[1] = 0;
+        if (grid)
+            NB_CUDA(cudaMemcpyAsync(status, grid_traj_status(grid_ws.get(), n), 2 * sizeof(int), cudaMemcpyDeviceToHost,
+                                    stream.get()));
+        rc = spin_wait(stream.get());
         if (rc) return rc;
-        memcpy(h_ev.data(), pin_ev, S * sizeof(nb_events));
-        if (pin_status[1] != 0) g_torn_records += pin_status[1];  // records that failed the full self-check and were fetched again
-        if (*pin_status != 0) {
+        memcpy(h_ev.data(), pin_ev.get(), S * sizeof(nb_events));
+        if (status[1] != 0) g_torn_records += status[1];  // records that failed the full self-check and were fetched again
+        if (status[0] != 0) {
             set_error_detail("grid trajectory kernel: exchange spin timed out (blocks not co-resident?)");
             return NB_ERR_CUDA;
         }
         float ms = 0;
-        NB_CUDA(cudaEventElapsedTime(&ms, e0, e1));
+        NB_CUDA(cudaEventElapsedTime(&ms, e0.get(), e1.get()));
         gpu_seconds += ms * 1e-3;
         for (int s = 0; s < S; s++) {
             long long steps = h_ev[s].steps_done - cur_step[s];
@@ -373,102 +342,102 @@ struct DeviceBatch {
         return NB_OK;
     }
     static bool stopped(const nb_events& e, int kind) { return kind >= NB_KIND_Q2 && e.hit_step != -2; }
+    // n > NB_MAX_SMALL_N: steps step0 + 1 .. step_end of the G systems s0 .. s0 + G - 1, stepped together, each step
+    // enqueued with its observers by enqueue_step(st).  Steps go out in chunks: while chunk c + 1 runs, the host reads the
+    // events after chunk c and enqueues nothing more once every system has stopped.  A step costs about G n^2 pairs (2.95 ms
+    // at G = 1, n = 65 536 on the B200), so a chunk is 2^33 / (G n^2) steps, at least 4 (~12 ms at 65 536 bodies) and at
+    // most 512 (below ~4 096 bodies a step is bound by launch latency).
+    template <class EnqueueStep>
+    int run_chunks(int s0, int G, int step0, int step_end, EnqueueStep enqueue_step) {
+        const int chunk = (int)std::min(512LL, std::max(4LL, (1LL << 33) / ((long long)G * n * n)));
+        for (int st = step0, c = 0; st < step_end; c++) {
+            for (const int end = std::min(st + chunk, step_end); st < end;) {
+                const int rc = enqueue_step(++st);
+                if (rc) return rc;
+            }
+            if (st >= step_end) break;
+            NB_CUDA(cudaMemcpyAsync(pin_chunk.get() + (size_t)(c & 1) * G, ev.get() + s0, G * sizeof(nb_events),
+                                    cudaMemcpyDeviceToHost, stream.get()));
+            NB_CUDA(cudaEventRecord(chunk_done[c & 1].get(), stream.get()));
+            if (c > 0) {  // chunk c is queued: read the events after chunk c - 1
+                const int rc = spin_wait(stream.get(), chunk_done[(c - 1) & 1].get());
+                if (rc) return rc;
+                const nb_events* prev = pin_chunk.get() + (size_t)((c - 1) & 1) * G;
+                bool all = true;
+                for (int g = 0; g < G && all; g++) all = stopped(prev[g], h_descs[s0 + g].kind);
+                if (all) break;
+            }
+        }
+        return NB_OK;
+    }
     // n > NB_MAX_SMALL_N: the systems one after another on the large-N steppers, each step followed by the one-warp observer
-    // (large_observe_kernel), step_begin observed first unless it already was.  Steps go out in chunks of large_chunk(n):
-    // while chunk c + 1 runs, the host reads the events after chunk c and enqueues nothing more once the stop event has
-    // fired.  The q, v left in a stopped slot are therefore up to two chunks past the stop, while cur_step (= steps_done) is
-    // the stop step: get_state would not return the state at cur_step there.  Nothing reads it - solve_chain reloads such
-    // a slot, and later runs skip a stopped system - so it is not rewound.
+    // (large_observe_kernel), step_begin observed first unless it already was.  The q, v left in a stopped slot are up to
+    // two chunks past the stop (run_chunks), while cur_step (= steps_done) is the stop step: get_state would not return the
+    // state at cur_step there.  Nothing reads it - solve_chain reloads such a slot, and later runs skip a stopped system -
+    // so it is not rewound.
     int run_large() {
-        const int chunk = large_chunk(n);
         for (int s = 0; s < S; s++) {
             const TrajDesc& d = h_descs[s];
             if (stopped(h_ev[s], d.kind) || h_ev[s].steps_done >= d.step_end) continue;
-            int rc = large.pack(d.q, d.m, d.is_device, d.step_begin + 1, stream);
-            if (!rc) rc = launch_large_observe(d, large.pos[large.cur], d.step_begin, stream);
-            for (int st = d.step_begin, c = 0; !rc && st < d.step_end; c++) {
-                const int end = std::min(st + chunk, d.step_end);
-                while (!rc && st < end) {
-                    rc = large.step(++st, d.v, d.m, d.is_device, stream);
-                    if (!rc) rc = launch_large_observe(d, large.pos[large.cur], st, stream);
-                }
-                if (rc || st >= d.step_end) break;
-                NB_CUDA(cudaMemcpyAsync(pin_chunk + (c & 1), d.ev, sizeof(nb_events), cudaMemcpyDeviceToHost, stream));
-                NB_CUDA(cudaEventRecord(chunk_done[c & 1], stream));
-                if (c > 0) {  // chunk c is queued: read the events after chunk c - 1
-                    rc = spin_wait(stream, chunk_done[(c - 1) & 1]);
-                    if (!rc && stopped(pin_chunk[(c - 1) & 1], d.kind)) break;
-                }
-            }
-            if (!rc) rc = large.unpack(d.q, stream);
+            int rc = large.pack(d.q, d.m, d.is_device, d.step_begin + 1, stream.get());
+            if (!rc) rc = launch_large_observe(d, large.pos[large.cur].get(), d.step_begin, stream.get());
+            if (!rc)
+                rc = run_chunks(s, 1, d.step_begin, d.step_end, [&](int st) {
+                    const int r = large.step(st, d.v, d.m, d.is_device, stream.get());
+                    return r ? r : launch_large_observe(d, large.pos[large.cur].get(), st, stream.get());
+                });
+            if (!rc) rc = large.unpack(d.q, stream.get());
             if (rc) return rc;
         }
         return NB_OK;
     }
     // Ensembles of n > NB_MAX_SMALL_N: every system starts at the same step.  The systems go in groups of G whose scratch fits
     // ENS_GROUP_BYTES; a group is packed (one nb_large_pack per system), its step_begin observed unless it already was, and
-    // stepped by three launches per step for all its systems (ens_step, ens_observe).  Steps go out in chunks as in
-    // run_large; the host reads the group's events after each chunk and enqueues nothing more once every member has stopped.
-    // A stopped member returns at the top of every kernel, so its records and v stay at its hit step, and each member is
-    // unpacked from the records of its own steps_done.
+    // stepped by three launches per step for all its systems (ens_step, ens_observe) until every member has stopped
+    // (run_chunks).  A stopped member returns at the top of every kernel, so its records and v stay at its hit step, and
+    // each member is unpacked from the records of its own steps_done.
     int run_ens_large() {
         const int n_pad = ens_pad(n), n_slots = ens_slots(math, n);
         const size_t per_sys = ((size_t)n_slots * 3 * sizeof(double) + 2 * sizeof(double4)) * n_pad;
         const int G_max = (int)std::max<size_t>(1, std::min<size_t>({(size_t)S, ENS_GROUP_BYTES / per_sys, 65535}));
         const int step0 = h_descs[0].step_begin, step_end = h_descs[0].step_end;
-        double4* pos4 = nullptr;
-        double* slots = nullptr;
-        NB_CUDA(cudaMalloc(&pos4, 2 * (size_t)G_max * n_pad * sizeof(double4)));
-        int rc = cuda_fail_or_ok(cudaMalloc(&slots, (size_t)G_max * n_slots * 3 * n_pad * sizeof(double)), "cudaMalloc slots");
+        DeviceMem<double4> pos4;
+        DeviceMem<double> slots;
+        NB_CUDA(alloc(pos4, 2 * (size_t)G_max * n_pad * sizeof(double4)));
+        NB_CUDA(alloc(slots, (size_t)G_max * n_slots * 3 * n_pad * sizeof(double)));
         // the records past n are zero (massless, at the origin) for good: nothing writes them
-        if (!rc) rc = cuda_fail_or_ok(cudaMemsetAsync(pos4, 0, 2 * (size_t)G_max * n_pad * sizeof(double4), stream), "memset");
-        for (int s0 = 0; s0 < S && !rc; s0 += G_max) {
-            const EnsGroup e{descs + s0, pos4, slots, n, n_pad, n_slots, std::min(G_max, S - s0)};
-            const long long work = (long long)e.G * n * n;
-            const int chunk = (int)std::min(512LL, std::max(4LL, (1LL << 33) / work));
+        NB_CUDA(cudaMemsetAsync(pos4.get(), 0, 2 * (size_t)G_max * n_pad * sizeof(double4), stream.get()));
+        for (int s0 = 0; s0 < S; s0 += G_max) {
+            const EnsGroup e{descs.get() + s0, pos4.get(), slots.get(), n, n_pad, n_slots, std::min(G_max, S - s0)};
+            auto rec = [&](int step, int g) { return (double*)(e.pos4 + ((size_t)(step & 1) * e.G + g) * n_pad); };
+            int rc = NB_OK;
             for (int g = 0; g < e.G && !rc; g++) {
                 const TrajDesc& d = h_descs[s0 + g];
-                double* rec = (double*)(pos4 + ((size_t)(step0 & 1) * e.G + g) * n_pad);
-                rc = nb_large_pack(math, n, d.q, d.m, d.is_device, step0 + 1, rec, stream);
+                rc = nb_large_pack(math, n, d.q, d.m, d.is_device, step0 + 1, rec(step0, g), stream.get());
             }
-            if (!rc) rc = ens_observe(e, step0, stream);
-            for (int st = step0, c = 0; !rc && st < step_end; c++) {
-                const int end = std::min(st + chunk, step_end);
-                while (!rc && st < end) {
-                    rc = ens_step(math, e, ++st, stream);
-                    if (!rc) rc = ens_observe(e, st, stream);
-                }
-                if (rc || st >= step_end) break;
-                nb_events* pin = pin_chunk + (size_t)(c & 1) * S;
-                rc = cuda_fail_or_ok(cudaMemcpyAsync(pin, ev + s0, e.G * sizeof(nb_events), cudaMemcpyDeviceToHost, stream),
-                                     "D2H chunk events");
-                if (!rc) rc = cuda_fail_or_ok(cudaEventRecord(chunk_done[c & 1], stream), "cudaEventRecord");
-                if (!rc && c > 0) {  // chunk c is queued: read the events after chunk c - 1
-                    rc = spin_wait(stream, chunk_done[(c - 1) & 1]);
-                    const nb_events* prev = pin_chunk + (size_t)((c - 1) & 1) * S;
-                    bool all = true;
-                    for (int g = 0; g < e.G && all; g++) all = stopped(prev[g], h_descs[s0 + g].kind);
-                    if (!rc && all) break;
-                }
-            }
+            if (!rc) rc = ens_observe(e, step0, stream.get());
+            if (!rc)
+                rc = run_chunks(s0, e.G, step0, step_end, [&](int st) {
+                    const int r = ens_step(math, e, st, stream.get());
+                    return r ? r : ens_observe(e, st, stream.get());
+                });
+            if (rc) return rc;
             // each member's records of its own last step
-            if (!rc) rc = cuda_fail_or_ok(cudaMemcpyAsync(pin_chunk, ev + s0, e.G * sizeof(nb_events), cudaMemcpyDeviceToHost,
-                                                          stream), "D2H group events");
-            if (!rc) rc = spin_wait(stream);
+            NB_CUDA(cudaMemcpyAsync(pin_chunk.get(), ev.get() + s0, e.G * sizeof(nb_events), cudaMemcpyDeviceToHost,
+                                    stream.get()));
+            rc = spin_wait(stream.get());
             for (int g = 0; g < e.G && !rc; g++)
-                rc = nb_large_unpack(n, (const double*)(pos4 + ((size_t)(pin_chunk[g].steps_done & 1) * e.G + g) * n_pad),
-                                     h_descs[s0 + g].q, stream);
+                rc = nb_large_unpack(n, rec(pin_chunk.get()[g].steps_done, g), h_descs[s0 + g].q, stream.get());
+            if (rc) return rc;
         }
-        if (!rc) rc = spin_wait(stream);
-        cudaFree(pos4), cudaFree(slots);
-        return rc;
+        return spin_wait(stream.get());
     }
     int get_state(int s, double* hq, double* hv, double* hm) {
         NB_CUDA(cudaSetDevice(gpu));
-        if (hq) NB_CUDA(cudaMemcpyAsync(hq, q + (size_t)s * 3 * n, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, stream));
-        if (hv) NB_CUDA(cudaMemcpyAsync(hv, v + (size_t)s * 3 * n, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, stream));
-        if (hm) NB_CUDA(cudaMemcpyAsync(hm, m + (size_t)s * n, n * sizeof(double), cudaMemcpyDeviceToHost, stream));
-        NB_CUDA(cudaStreamSynchronize(stream));
+        if (hq) NB_CUDA(cudaMemcpyAsync(hq, q.get() + (size_t)s * 3 * n, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, stream.get()));
+        if (hv) NB_CUDA(cudaMemcpyAsync(hv, v.get() + (size_t)s * 3 * n, 3 * n * sizeof(double), cudaMemcpyDeviceToHost, stream.get()));
+        if (hm) NB_CUDA(cudaMemcpyAsync(hm, m.get() + (size_t)s * n, n * sizeof(double), cudaMemcpyDeviceToHost, stream.get()));
+        NB_CUDA(cudaStreamSynchronize(stream.get()));
         return NB_OK;
     }
 };
@@ -542,18 +511,14 @@ int nb_traj_create(int gpu, const nb_system* sys, int kind, int destroy_device, 
     if (kind < NB_KIND_PLAIN || kind > NB_KIND_Q3 || (math != NB_MATH_FAST && math != NB_MATH_STRICT)) return NB_ERR_ARG;
     int rc = nb::check_gpu(gpu);
     if (rc) return rc;
-    nb_traj* t = new nb_traj();
+    std::unique_ptr<nb_traj> t(new nb_traj());
     t->planet = sys->planet, t->asteroid = sys->asteroid, t->kind = kind, t->destroy_device = destroy_device;
     t->isdev.assign(sys->is_device, sys->is_device + sys->n);
     rc = t->b.init(gpu, 1, sys->n, math);
     if (!rc)
         rc = t->b.set_system(0, sys->q, sys->v, sys->m, sys->is_device, sys->planet, sys->asteroid, kind, destroy_device, 0);
-    if (rc) {
-        t->b.release();
-        delete t;
-        return rc;
-    }
-    *out = t;
+    if (rc) return rc;
+    *out = t.release();
     return NB_OK;
 }
 
@@ -583,32 +548,25 @@ int nb_traj_fork_on(nb_traj* t, int gpu, int kind, int destroy_device, nb_traj**
     std::vector<double> m(n);
     rc = t->b.get_state(0, nullptr, nullptr, m.data());
     if (rc) return rc;
-    nb_traj* f = new nb_traj();
+    std::unique_ptr<nb_traj> f(new nb_traj());
     f->planet = t->planet, f->asteroid = t->asteroid, f->kind = kind, f->destroy_device = destroy_device;
     f->isdev = t->isdev;
     rc = f->b.init(gpu, 1, n, t->b.math);
     if (!rc)
         rc = f->b.set_system(0, nullptr, nullptr, m.data(), f->isdev.data(), f->planet, f->asteroid, kind, destroy_device,
                              t->b.cur_step[0]);
-    if (!rc) {
-        const size_t bytes = 3 * (size_t)n * sizeof(double);
-        cudaError_t e = cudaSuccess;
-        if (gpu == t->b.gpu) {
-            e = cudaMemcpyAsync(f->b.q, t->b.q, bytes, cudaMemcpyDeviceToDevice, f->b.stream);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(f->b.v, t->b.v, bytes, cudaMemcpyDeviceToDevice, f->b.stream);
-        } else {
-            e = cudaMemcpyPeerAsync(f->b.q, gpu, t->b.q, t->b.gpu, bytes, f->b.stream);
-            if (e == cudaSuccess) e = cudaMemcpyPeerAsync(f->b.v, gpu, t->b.v, t->b.gpu, bytes, f->b.stream);
-        }
-        if (e == cudaSuccess) e = cudaStreamSynchronize(f->b.stream);
-        if (e != cudaSuccess) rc = nb::cuda_fail(e, "fork copy", __FILE__, __LINE__);
+    if (rc) return rc;
+    const size_t bytes = 3 * (size_t)n * sizeof(double);
+    cudaStream_t st = f->b.stream.get();
+    if (gpu == t->b.gpu) {
+        NB_CUDA(cudaMemcpyAsync(f->b.q.get(), t->b.q.get(), bytes, cudaMemcpyDeviceToDevice, st));
+        NB_CUDA(cudaMemcpyAsync(f->b.v.get(), t->b.v.get(), bytes, cudaMemcpyDeviceToDevice, st));
+    } else {
+        NB_CUDA(cudaMemcpyPeerAsync(f->b.q.get(), gpu, t->b.q.get(), t->b.gpu, bytes, st));
+        NB_CUDA(cudaMemcpyPeerAsync(f->b.v.get(), gpu, t->b.v.get(), t->b.gpu, bytes, st));
     }
-    if (rc) {
-        f->b.release();
-        delete f;
-        return rc;
-    }
-    *out = f;
+    NB_CUDA(cudaStreamSynchronize(st));
+    *out = f.release();
     return NB_OK;
 }
 
@@ -619,20 +577,34 @@ int nb_traj_fork(nb_traj* t, int kind, int destroy_device, nb_traj** out) {
 
 int nb_traj_destroy(nb_traj* t) {
     if (!t) return NB_ERR_ARG;
-    t->b.release();
     delete t;
     return NB_OK;
 }
 
 // ---- diagnostics (nb_diag.cu) ---------------------------------------------------------------------------
-// [S][9] device results -> nb_diag
-static void diag_unpack(const double* r, int S, int n, int step, nb_diag* out) {
+// S systems whose arrays are on the device, with the masses of `step`, on stream st; e0 / e1, when given, bracket the
+// kernels.  Returns once out[S] is filled.
+static int diag_run(int S, int n, const double* q, const double* v, const double* m, const unsigned char* is_device,
+                    int step, cudaStream_t st, nb_diag* out, cudaEvent_t e0 = nullptr, cudaEvent_t e1 = nullptr) {
+    nb::DeviceMem<void> scratch;
+    nb::DeviceMem<double> dout;
+    std::vector<double> res((size_t)S * 9);  // [S][9] {mass, kinetic, potential, P[3], L[3]}
+    NB_CUDA(nb::alloc(scratch, nb::diag_scratch_bytes(S, n)));
+    NB_CUDA(nb::alloc(dout, res.size() * sizeof(double)));
+    if (e0) NB_CUDA(cudaEventRecord(e0, st));
+    const int rc = nb::diag_launch(S, n, q, v, m, is_device, nb::fst_at(step), scratch.get(), dout.get(), st);
+    if (rc) return rc;
+    if (e1) NB_CUDA(cudaEventRecord(e1, st));
+    NB_CUDA(cudaMemcpyAsync(res.data(), dout.get(), res.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+    NB_CUDA(cudaStreamSynchronize(st));
+    const double* r = res.data();
     for (int s = 0; s < S; s++, r += 9) {
         nb_diag& d = out[s];
         d.step = step, d.n = n;
         d.mass = r[0], d.kinetic = r[1], d.potential = r[2];
         for (int c = 0; c < 3; c++) d.momentum[c] = r[3 + c], d.angular_momentum[c] = r[6 + c];
     }
+    return NB_OK;
 }
 
 int nb_diagnostics(int gpu, int n_systems, int n, const double* q, const double* v, const double* m,
@@ -642,73 +614,35 @@ int nb_diagnostics(int gpu, int n_systems, int n, const double* q, const double*
     if (rc) return rc;
     NB_CUDA(cudaSetDevice(gpu));
     const size_t S = (size_t)n_systems, qb = S * 3 * n * sizeof(double);
-    cudaStream_t st = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    double *dq = nullptr, *dv = nullptr, *dm = nullptr, *dout = nullptr;
-    unsigned char* ddev = nullptr;
-    void* scratch = nullptr;
-    std::vector<double> res(S * 9);
-    auto chk = [&](cudaError_t e, const char* what) {
-        if (e != cudaSuccess && rc == NB_OK) rc = nb::cuda_fail(e, what, __FILE__, __LINE__);
-    };
-    chk(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking), "cudaStreamCreate");
-    chk(cudaEventCreate(&e0), "cudaEventCreate");
-    chk(cudaEventCreate(&e1), "cudaEventCreate");
-    chk(cudaMalloc(&dq, qb), "cudaMalloc q");
-    chk(cudaMalloc(&dv, qb), "cudaMalloc v");
-    chk(cudaMalloc(&dm, S * n * sizeof(double)), "cudaMalloc m");
-    chk(cudaMalloc(&ddev, S * n), "cudaMalloc is_device");
-    chk(cudaMalloc(&dout, S * 9 * sizeof(double)), "cudaMalloc out");
-    chk(cudaMalloc(&scratch, nb::diag_scratch_bytes(n_systems, n)), "cudaMalloc scratch");
-    if (rc == NB_OK) {
-        chk(cudaMemcpyAsync(dq, q, qb, cudaMemcpyHostToDevice, st), "H2D q");
-        chk(cudaMemcpyAsync(dv, v, qb, cudaMemcpyHostToDevice, st), "H2D v");
-        chk(cudaMemcpyAsync(dm, m, S * n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D m");
-        chk(cudaMemcpyAsync(ddev, is_device, S * n, cudaMemcpyHostToDevice, st), "H2D is_device");
-        chk(cudaEventRecord(e0, st), "cudaEventRecord");
-    }
-    if (rc == NB_OK) rc = nb::diag_launch(n_systems, n, dq, dv, dm, ddev, nb::fst_at(step), scratch, dout, st);
-    if (rc == NB_OK) {
-        chk(cudaEventRecord(e1, st), "cudaEventRecord");
-        chk(cudaMemcpyAsync(res.data(), dout, S * 9 * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H out");
-        chk(cudaStreamSynchronize(st), "sync");
-    }
-    if (rc == NB_OK) {
-        float ms = 0;
-        chk(cudaEventElapsedTime(&ms, e0, e1), "cudaEventElapsedTime");
-        if (gpu_seconds) *gpu_seconds = ms * 1e-3;
-        diag_unpack(res.data(), n_systems, n, step, out);
-    }
-    cudaFree(dq), cudaFree(dv), cudaFree(dm), cudaFree(ddev), cudaFree(dout), cudaFree(scratch);
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    if (st) cudaStreamDestroy(st);
-    return rc;
+    nb::Stream st;
+    nb::Event e0, e1;
+    nb::DeviceMem<double> dq, dv, dm;
+    nb::DeviceMem<unsigned char> ddev;
+    NB_CUDA(nb::create(st));
+    NB_CUDA(nb::create(e0));
+    NB_CUDA(nb::create(e1));
+    NB_CUDA(nb::alloc(dq, qb));
+    NB_CUDA(nb::alloc(dv, qb));
+    NB_CUDA(nb::alloc(dm, S * n * sizeof(double)));
+    NB_CUDA(nb::alloc(ddev, S * n));
+    NB_CUDA(cudaMemcpyAsync(dq.get(), q, qb, cudaMemcpyHostToDevice, st.get()));
+    NB_CUDA(cudaMemcpyAsync(dv.get(), v, qb, cudaMemcpyHostToDevice, st.get()));
+    NB_CUDA(cudaMemcpyAsync(dm.get(), m, S * n * sizeof(double), cudaMemcpyHostToDevice, st.get()));
+    NB_CUDA(cudaMemcpyAsync(ddev.get(), is_device, S * n, cudaMemcpyHostToDevice, st.get()));
+    rc = diag_run(n_systems, n, dq.get(), dv.get(), dm.get(), ddev.get(), step, st.get(), out, e0.get(), e1.get());
+    if (rc) return rc;
+    float ms = 0;
+    NB_CUDA(cudaEventElapsedTime(&ms, e0.get(), e1.get()));
+    if (gpu_seconds) *gpu_seconds = ms * 1e-3;
+    return NB_OK;
 }
 
 // slot 0 of the handle's batch, on its stream: q, v stay on the device
 int nb_traj_diagnostics(nb_traj* t, nb_diag* out) {
     if (!t || !out) return NB_ERR_ARG;
-    DeviceBatch& b = t->b;
+    const DeviceBatch& b = t->b;
     NB_CUDA(cudaSetDevice(b.gpu));
-    const int n = b.n, step = b.cur_step[0];
-    void* scratch = nullptr;
-    double* dout = nullptr;
-    double res[9];
-    int rc = NB_OK;
-    auto chk = [&](cudaError_t e, const char* what) {
-        if (e != cudaSuccess && rc == NB_OK) rc = nb::cuda_fail(e, what, __FILE__, __LINE__);
-    };
-    chk(cudaMalloc(&scratch, nb::diag_scratch_bytes(1, n)), "cudaMalloc scratch");
-    chk(cudaMalloc(&dout, 9 * sizeof(double)), "cudaMalloc out");
-    if (rc == NB_OK) rc = nb::diag_launch(1, n, b.q, b.v, b.m, b.isdev, nb::fst_at(step), scratch, dout, b.stream);
-    if (rc == NB_OK) {
-        chk(cudaMemcpyAsync(res, dout, sizeof res, cudaMemcpyDeviceToHost, b.stream), "D2H out");
-        chk(cudaStreamSynchronize(b.stream), "sync");
-    }
-    if (rc == NB_OK) diag_unpack(res, 1, n, step, out);
-    cudaFree(scratch), cudaFree(dout);
-    return rc;
+    return diag_run(1, b.n, b.q.get(), b.v.get(), b.m.get(), b.isdev.get(), b.cur_step[0], b.stream.get(), out);
 }
 
 // ---- ensembles ---------------------------------------------------------------------------------------
@@ -727,60 +661,50 @@ int nb_ensemble_run(int gpu, int math, int kind, int n_systems, int n, double* q
         rc = b.set_system(s, q + (size_t)s * 3 * n, v + (size_t)s * 3 * n, m + (size_t)s * n, is_device + (size_t)s * n,
                           planet ? planet[s] : 0, asteroid ? asteroid[s] : 0, kind,
                           destroy_device ? destroy_device[s] : -1, step_begin);
-    if (!rc && step_begin > 0) {
+    if (rc) return rc;
+    if (step_begin > 0) {
         // resuming: the caller has observed step_begin already
         for (int s = 0; s < n_systems; s++) b.h_ev[s].steps_done = step_begin;
-        cudaError_t e = cudaMemcpy(b.ev, b.h_ev.data(), n_systems * sizeof(nb_events), cudaMemcpyHostToDevice);
-        if (e != cudaSuccess) rc = nb::cuda_fail(e, "cudaMemcpy(ev)", __FILE__, __LINE__);
+        NB_CUDA(cudaMemcpy(b.ev.get(), b.h_ev.data(), n_systems * sizeof(nb_events), cudaMemcpyHostToDevice));
     }
-    if (!rc) rc = b.run(step_end, false);
+    rc = b.run(step_end, false);
     for (int s = 0; s < n_systems && !rc; s++) {
         rc = b.get_state(s, q + (size_t)s * 3 * n, v + (size_t)s * 3 * n, nullptr);
         if (ev) ev[s] = b.h_ev[s];
     }
     if (gpu_seconds) *gpu_seconds = b.gpu_seconds;
-    b.release();
     return rc;
 }
 
 // ---- the step operator -------------------------------------------------------------------------------
-// n > NB_MAX_SMALL_N on one GPU (LargeStepper), host buffers in and out.  The first failing call's code is returned;
-// everything is freed on every path.
+// n > NB_MAX_SMALL_N on one GPU (LargeStepper), host buffers in and out
 static int run_steps_large(int gpu, int math, int n, double* q, double* v, const double* m, const unsigned char* is_device,
                            int step_begin, int step_end) {
     NB_CUDA(cudaSetDevice(gpu));
-    int rc = NB_OK;
-    cudaStream_t st = nullptr;
-    double *dq = nullptr, *dv = nullptr, *dm = nullptr;
-    unsigned char* ddev = nullptr;
+    const size_t qb = 3 * (size_t)n * sizeof(double);
+    nb::Stream st;
+    nb::DeviceMem<double> dq, dv, dm;
+    nb::DeviceMem<unsigned char> ddev;
     nb::LargeStepper ls;
-    auto chk = [&](cudaError_t e, const char* what) {
-        if (e != cudaSuccess && rc == NB_OK) rc = nb::cuda_fail(e, what, __FILE__, __LINE__);
-    };
-    chk(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking), "cudaStreamCreate");
-    chk(cudaMalloc(&dq, 3 * (size_t)n * sizeof(double)), "cudaMalloc q");
-    chk(cudaMalloc(&dv, 3 * (size_t)n * sizeof(double)), "cudaMalloc v");
-    chk(cudaMalloc(&dm, (size_t)n * sizeof(double)), "cudaMalloc m");
-    chk(cudaMalloc(&ddev, (size_t)n), "cudaMalloc is_device");
-    if (rc == NB_OK) rc = ls.init(n, math, st);
-    if (rc == NB_OK) {
-        chk(cudaMemcpyAsync(dq, q, 3 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D q");
-        chk(cudaMemcpyAsync(dv, v, 3 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D v");
-        chk(cudaMemcpyAsync(dm, m, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st), "H2D m");
-        chk(cudaMemcpyAsync(ddev, is_device, (size_t)n, cudaMemcpyHostToDevice, st), "H2D is_device");
-    }
-    if (rc == NB_OK) rc = ls.pack(dq, dm, ddev, step_begin + 1, st);
-    for (int step = step_begin + 1; step <= step_end && rc == NB_OK; step++) rc = ls.step(step, dv, dm, ddev, st);
-    if (rc == NB_OK) rc = ls.unpack(dq, st);
-    if (rc == NB_OK) {
-        chk(cudaMemcpyAsync(q, dq, 3 * (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H q");
-        chk(cudaMemcpyAsync(v, dv, 3 * (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st), "D2H v");
-        chk(cudaStreamSynchronize(st), "sync");
-    }
-    cudaFree(dq), cudaFree(dv), cudaFree(dm), cudaFree(ddev);
-    ls.release();
-    if (st) cudaStreamDestroy(st);
-    return rc;
+    NB_CUDA(nb::create(st));
+    NB_CUDA(nb::alloc(dq, qb));
+    NB_CUDA(nb::alloc(dv, qb));
+    NB_CUDA(nb::alloc(dm, (size_t)n * sizeof(double)));
+    NB_CUDA(nb::alloc(ddev, (size_t)n));
+    int rc = ls.init(n, math, st.get());
+    if (rc) return rc;
+    NB_CUDA(cudaMemcpyAsync(dq.get(), q, qb, cudaMemcpyHostToDevice, st.get()));
+    NB_CUDA(cudaMemcpyAsync(dv.get(), v, qb, cudaMemcpyHostToDevice, st.get()));
+    NB_CUDA(cudaMemcpyAsync(dm.get(), m, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st.get()));
+    NB_CUDA(cudaMemcpyAsync(ddev.get(), is_device, (size_t)n, cudaMemcpyHostToDevice, st.get()));
+    rc = ls.pack(dq.get(), dm.get(), ddev.get(), step_begin + 1, st.get());
+    for (int step = step_begin + 1; step <= step_end && !rc; step++) rc = ls.step(step, dv.get(), dm.get(), ddev.get(), st.get());
+    if (!rc) rc = ls.unpack(dq.get(), st.get());
+    if (rc) return rc;
+    NB_CUDA(cudaMemcpyAsync(q, dq.get(), qb, cudaMemcpyDeviceToHost, st.get()));
+    NB_CUDA(cudaMemcpyAsync(v, dv.get(), qb, cudaMemcpyDeviceToHost, st.get()));
+    NB_CUDA(cudaStreamSynchronize(st.get()));
+    return NB_OK;
 }
 
 int nb_run_steps(int gpu, int math, int n, double* q, double* v, const double* m, const unsigned char* is_device,
@@ -795,7 +719,6 @@ int nb_run_steps(int gpu, int math, int n, double* q, double* v, const double* m
     if (!rc) rc = b.set_system(0, q, v, m, is_device, 0, 0, NB_KIND_PLAIN, -1, step_begin);
     if (!rc) rc = b.run(step_end, true);
     if (!rc) rc = b.get_state(0, q, v, nullptr);
-    b.release();
     return rc;
 }
 
@@ -869,6 +792,11 @@ static int solve_chain(const nb_system* sys, const std::vector<int>& devs, const
     const size_t sbytes = 3 * (size_t)n * sizeof(double);
     int rc = nb::check_gpu(gpu);
     if (rc) return rc;
+    // lag = Q2's q, v at the start of the current chunk; snap[k] = fork point of device k: q, v at the start of the chunk
+    // its missile arrived in.  Both are declared before b, so they are freed after b's destructor has made gpu current.
+    nb::DeviceMem<double> lag;
+    std::vector<nb::DeviceMem<double>> snap(dc);
+    std::vector<int> snap_step(dc, -1);
     DeviceBatch b;
     const int S = (with_q1 ? 1 : 0) + (with_chain ? 1 : 0), sl = S - 1;  // sl = slot of the chain
     const auto t_init = std::chrono::steady_clock::now();
@@ -879,28 +807,16 @@ static int solve_chain(const nb_system* sys, const std::vector<int>& devs, const
     if (!rc && with_q1) rc = b.set_system(0, sys->q, sys->v, sys->m, sys->is_device, sys->planet, sys->asteroid, NB_KIND_Q1, -1, 0);
     if (!rc && with_chain)
         rc = b.set_system(sl, sys->q, sys->v, sys->m, sys->is_device, sys->planet, sys->asteroid, NB_KIND_Q2, -1, 0);
-    double* lag = nullptr;               // Q2's q, v at the start of the current chunk
-    std::vector<double*> snap(dc, nullptr);  // fork point of device k: q, v at the start of the chunk its missile arrived in
-    std::vector<int> snap_step(dc, -1);
-    auto cleanup = [&](int r) {
-        if (nb::g_leak_on_exit.load()) return r;
-        cudaSetDevice(gpu);
-        if (lag) cudaFree(lag);
-        for (double* p : snap)
-            if (p) cudaFree(p);
-        b.release();
-        return r;
-    };
-    if (rc) return cleanup(rc);
+    if (rc) return rc;
     int n_launch = 0;
     const auto t_run = std::chrono::steady_clock::now();
     if (!with_chain) {
         rc = b.run(n_steps, true);
         if (!rc) evs[0] = b.h_ev[0];
     } else {
-        if (cudaMalloc(&lag, 2 * sbytes) != cudaSuccess) return cleanup(NB_ERR_CUDA);
-        double* cq = b.q + (size_t)sl * 3 * n;
-        double* cv = b.v + (size_t)sl * 3 * n;
+        NB_CUDA(nb::alloc(lag, 2 * sbytes));
+        double* cq = b.q.get() + (size_t)sl * 3 * n;
+        double* cv = b.v.get() + (size_t)sl * 3 * n;
         // ---- Q2 (and Q1 beside it), chunk by chunk while a missile is still under way
         int cur = 0;
         bool first = true;  // n_steps == 0 still observes step 0
@@ -912,9 +828,8 @@ static int solve_chain(const nb_system* sys, const std::vector<int>& devs, const
             // steps pair with the Q3 candidate's in one launch
             const int next = cur + NB_SOLVE_CHUNK < n_steps ? cur + NB_SOLVE_CHUNK : n_steps;
             if (pending) {
-                if (cudaMemcpyAsync(lag, cq, sbytes, cudaMemcpyDeviceToDevice, b.stream) != cudaSuccess ||
-                    cudaMemcpyAsync(lag + 3 * n, cv, sbytes, cudaMemcpyDeviceToDevice, b.stream) != cudaSuccess)
-                    return cleanup(NB_ERR_CUDA);
+                NB_CUDA(cudaMemcpyAsync(lag.get(), cq, sbytes, cudaMemcpyDeviceToDevice, b.stream.get()));
+                NB_CUDA(cudaMemcpyAsync(lag.get() + 3 * n, cv, sbytes, cudaMemcpyDeviceToDevice, b.stream.get()));
             }
             const double g_before = b.gpu_seconds;
             rc = b.run(next, true);
@@ -922,14 +837,13 @@ static int solve_chain(const nb_system* sys, const std::vector<int>& devs, const
             if (verbose) fprintf(stderr, "nbody_b200:   Q2 chunk %d -> %d: kernels %.4f s\n", cur, next, b.gpu_seconds - g_before);
             for (int k = 0; k < dc && !rc; k++)
                 if (snap_step[k] < 0 && b.h_ev[sl].reach_step[k] != -2) {
-                    if (cudaMalloc(&snap[k], 2 * sbytes) != cudaSuccess ||
-                        cudaMemcpyAsync(snap[k], lag, 2 * sbytes, cudaMemcpyDeviceToDevice, b.stream) != cudaSuccess)
-                        return cleanup(NB_ERR_CUDA);
+                    NB_CUDA(nb::alloc(snap[k], 2 * sbytes));
+                    NB_CUDA(cudaMemcpyAsync(snap[k].get(), lag.get(), 2 * sbytes, cudaMemcpyDeviceToDevice, b.stream.get()));
                     snap_step[k] = cur;
                 }
             cur = next;
         }
-        if (rc) return cleanup(rc);
+        if (rc) return rc;
         evs[1] = b.h_ev[sl];
         for (int k = 0; k < dc; k++) {  // "not simulated" until tried; a speculated device is another part's entry
             DeviceBatch::fresh_events(evs[2 + k]);
@@ -945,16 +859,15 @@ static int solve_chain(const nb_system* sys, const std::vector<int>& devs, const
             for (int k : order) {
                 rc = b.set_system(sl, nullptr, nullptr, sys->m, sys->is_device, sys->planet, sys->asteroid, NB_KIND_Q3, devs[k],
                                   snap_step[k]);
-                if (rc) return cleanup(rc);
-                if (cudaMemcpyAsync(cq, snap[k], sbytes, cudaMemcpyDeviceToDevice, b.stream) != cudaSuccess ||
-                    cudaMemcpyAsync(cv, snap[k] + 3 * n, sbytes, cudaMemcpyDeviceToDevice, b.stream) != cudaSuccess)
-                    return cleanup(NB_ERR_CUDA);
+                if (rc) return rc;
+                NB_CUDA(cudaMemcpyAsync(cq, snap[k].get(), sbytes, cudaMemcpyDeviceToDevice, b.stream.get()));
+                NB_CUDA(cudaMemcpyAsync(cv, snap[k].get() + 3 * n, sbytes, cudaMemcpyDeviceToDevice, b.stream.get()));
                 const double g_before = b.gpu_seconds;
                 rc = b.run(n_steps, true);  // Q1, if still under way, rides along in the same launch
                 n_launch++;
                 if (verbose)
                     fprintf(stderr, "nbody_b200:   Q3 device %d from step %d: kernels %.4f s\n", devs[k], snap_step[k], b.gpu_seconds - g_before);
-                if (rc) return cleanup(rc);
+                if (rc) return rc;
                 evs[2 + k] = b.h_ev[sl];
                 if (b.h_ev[sl].hit_step == -2 && b.h_ev[sl].destroyed_step != -2) break;  // saved: the rest cost more
             }
@@ -974,7 +887,7 @@ static int solve_chain(const nb_system* sys, const std::vector<int>& devs, const
                 std::chrono::duration<double>(std::chrono::steady_clock::now() - t_run).count(), b.gpu_seconds);
     if (gpu_seconds) *gpu_seconds = b.gpu_seconds;
     if (pair_interactions) *pair_interactions = b.pairs;
-    return cleanup(rc);
+    return rc;
 }
 
 int nb_solve_partial(const nb_system* sys, int gpu, int part, int n_parts, int n_steps, int math, nb_events* evs,
@@ -1038,7 +951,6 @@ int nb_solve_partial(const nb_system* sys, int gpu, int part, int n_parts, int n
         for (size_t s = 0; s < mine.size(); s++) evs[mine[s]] = b.h_ev[s];
     if (gpu_seconds) *gpu_seconds = b.gpu_seconds;
     if (pair_interactions) *pair_interactions = b.pairs;
-    b.release();
     return rc;
 }
 

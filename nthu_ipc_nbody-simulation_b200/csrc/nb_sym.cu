@@ -522,10 +522,10 @@ using namespace nb::sym;
 struct nb_sym {
     Plan plan;
     int gpu = -1, integrate_blocks = 0;
-    Seg* d_segs = nullptr;
-    int *d_bsb = nullptr, *d_tables = nullptr;  // tables: pi_ptr | pi_list | pj_ptr | pj_list
+    DeviceMem<Seg> d_segs;
+    DeviceMem<int> d_bsb, d_tables;  // tables: pi_ptr | pi_list | pj_ptr | pj_list
     int off_pi_list = 0, off_pj_ptr = 0, off_pj_list = 0;
-    double* d_pi = nullptr;
+    DeviceMem<double> d_pi;
     long long steps_done[2] = {0, 0};  // steps executed per parity
     long long pos_pubs[2] = {0, 0};    // publications of this rank's rows per parity (integrate kernels + nb_sym_publish_rows)
     int first_step = -1, last_step = -1, accel_step = -1;
@@ -603,12 +603,9 @@ int nb_sym_create(int n, int world, int rank, nb_sym** out) {
     int blocks = 0;
     int rc = sym_default_blocks(&blocks);
     if (rc) return rc;
-    nb_sym* h = new nb_sym();
+    std::unique_ptr<nb_sym> h(new nb_sym());
     rc = build_plan(n, world, rank, blocks, choose_ipl(n, world), h->plan);
-    if (rc) {
-        delete h;
-        return rc;
-    }
+    if (rc) return rc;
     const Plan& P = h->plan;
     cudaGetDevice(&h->gpu);
     h->integrate_blocks = (P.shard + IB - 1) / IB;
@@ -621,30 +618,20 @@ int nb_sym_create(int n, int world, int rank, nb_sym** out) {
     h->off_pj_list = (int)tables.size();
     tables.insert(tables.end(), P.pj_list.begin(), P.pj_list.end());
     tables.push_back(0);
-    cudaError_t e = cudaSuccess;
-    auto ok = [&](cudaError_t x) {
-        if (e == cudaSuccess) e = x;
-    };
-    ok(cudaMalloc(&h->d_segs, std::max<size_t>(1, P.segs.size()) * sizeof(Seg)));
-    ok(cudaMalloc(&h->d_bsb, (blocks + 1) * sizeof(int)));
-    ok(cudaMalloc(&h->d_tables, tables.size() * sizeof(int)));
-    ok(cudaMalloc(&h->d_pi, std::max<size_t>(1, (size_t)P.pi_slots) * 3 * P.sb * sizeof(double)));
-    if (e == cudaSuccess && !P.segs.empty())
-        ok(cudaMemcpy(h->d_segs, P.segs.data(), P.segs.size() * sizeof(Seg), cudaMemcpyHostToDevice));
-    if (e == cudaSuccess) ok(cudaMemcpy(h->d_bsb, P.block_seg_begin.data(), (blocks + 1) * sizeof(int), cudaMemcpyHostToDevice));
-    if (e == cudaSuccess) ok(cudaMemcpy(h->d_tables, tables.data(), tables.size() * sizeof(int), cudaMemcpyHostToDevice));
-    if (e != cudaSuccess) {
-        rc = cuda_fail(e, "nb_sym_create", __FILE__, __LINE__);
-        nb_sym_destroy(h);
-        return rc;
-    }
-    *out = h;
+    NB_CUDA(alloc(h->d_segs, std::max<size_t>(1, P.segs.size()) * sizeof(Seg)));
+    NB_CUDA(alloc(h->d_bsb, (blocks + 1) * sizeof(int)));
+    NB_CUDA(alloc(h->d_tables, tables.size() * sizeof(int)));
+    NB_CUDA(alloc(h->d_pi, std::max<size_t>(1, (size_t)P.pi_slots) * 3 * P.sb * sizeof(double)));
+    if (!P.segs.empty())
+        NB_CUDA(cudaMemcpy(h->d_segs.get(), P.segs.data(), P.segs.size() * sizeof(Seg), cudaMemcpyHostToDevice));
+    NB_CUDA(cudaMemcpy(h->d_bsb.get(), P.block_seg_begin.data(), (blocks + 1) * sizeof(int), cudaMemcpyHostToDevice));
+    NB_CUDA(cudaMemcpy(h->d_tables.get(), tables.data(), tables.size() * sizeof(int), cudaMemcpyHostToDevice));
+    *out = h.release();
     return NB_OK;
 }
 
 int nb_sym_destroy(nb_sym* h) {
     if (!h) return NB_ERR_ARG;
-    cudaFree(h->d_segs), cudaFree(h->d_bsb), cudaFree(h->d_tables), cudaFree(h->d_pi);
     delete h;
     return NB_OK;
 }
@@ -701,7 +688,7 @@ int nb_sym_step_phase(nb_sym* h, int step, int phases, const double* pos4_cur, d
     cudaStream_t st = (cudaStream_t)stream;
     AccelArgs A{};
     A.pos4 = (const double4*)pos4_cur;
-    A.segs = h->d_segs, A.block_seg_begin = h->d_bsb, A.pi = h->d_pi, A.shard = P.shard;
+    A.segs = h->d_segs.get(), A.block_seg_begin = h->d_bsb.get(), A.pi = h->d_pi.get(), A.shard = P.shard;
     A.parity_read = (step - 1) & 1;
     // rows of step-1 were published by the integrate kernels of step-1 (none before the first step: packed locally)
     A.pos_target = P.world > 1 ? (unsigned long long)h->integrate_blocks * h->pos_pubs[(step - 1) & 1] : 0;
@@ -730,9 +717,9 @@ int nb_sym_step_phase(nb_sym* h, int step, int phases, const double* pos4_cur, d
     if (!(phases & 2)) return NB_OK;
     IntegrateArgs I{};
     I.pos4 = (const double4*)pos4_cur, I.vel = vel_dev, I.m0 = m0_dev, I.is_device = is_device_dev;
-    I.pi = h->d_pi, I.pj = peer_pj[P.rank];
-    I.pi_ptr = h->d_tables, I.pi_list = h->d_tables + h->off_pi_list;
-    I.pj_ptr = h->d_tables + h->off_pj_ptr, I.pj_list = h->d_tables + h->off_pj_list;
+    I.pi = h->d_pi.get(), I.pj = peer_pj[P.rank];
+    I.pi_ptr = h->d_tables.get(), I.pi_list = h->d_tables.get() + h->off_pi_list;
+    I.pj_ptr = h->d_tables.get() + h->off_pj_ptr, I.pj_list = h->d_tables.get() + h->off_pj_list;
     I.shard = P.shard, I.i_begin = P.rank * P.shard, I.row_stride = P.row_stride, I.sb = P.sb;
     I.fst_next = fst_value(step + 1);
     I.parity = step & 1;

@@ -19,7 +19,7 @@ pytestmark = pytest.mark.gpu
 MIN_DIST_RTOL = 1e-6
 PADDED = [("b20", 1025), ("b100", 1025), ("b512", 1500), ("b1024", 2048)]
 STEPS = 1000  # horizon of the constructed systems
-MAX_CHUNK = 512  # largest chunk of steps DeviceBatch::run_large enqueues between two reads of the events (large_chunk)
+MAX_CHUNK = 512  # largest chunk of steps DeviceBatch::run_large enqueues between two reads of the events (run_chunks)
 
 
 @pytest.fixture(scope="module")
